@@ -58,7 +58,37 @@ def parse():
                     help="fused arm: skip timing our NCCL+cuBLAS baseline in the same process (vs_baseline = null)")
     ap.add_argument("--two-shot", default="auto", choices=["auto", "on", "off"],
                     help="fused arm: FedAvg as reduce-own-slice + multicast publish (auto: by model size)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed round computed (global model + round result) "
+                         "as DIR/<name>.npy; the inputs are seeded, so two builds compare output for output")
     return ap.parse_args()
+
+
+DUMP_MAX_ELEMS = 1 << 21     # per array (8 MB of fp32): a dump of the MLP's four tensors stays < 64 MB
+
+
+def round_outputs(eng) -> dict:
+    """What a caller of the timed round receives: the global model (fp32, per tensor) and the
+    round's result (epoch, roles, global loss; the fused engine's ledger page adds the committee's
+    median scores and the FedAvg selection mask).  An array above DUMP_MAX_ELEMS is replaced by a
+    fixed, seeded sample of its elements."""
+    import numpy as np
+
+    if hasattr(eng, "global_master"):          # FusedEngine: replicated ledger page on the device
+        st = eng.read_state()
+        model = eng.spec.views(eng.global_master)
+        res = dict(epoch=st["epoch"], roles=st["roles"], median_scores=st["median"],
+                   selected_mask=st["selected_mask"], global_loss=st["global_loss"])
+    else:                                      # NcclBaselineEngine: host copy of the round's result
+        model = eng.spec.views(eng.global_w)
+        res = dict(epoch=eng.epoch, roles=eng.roles, global_loss=eng.global_loss)
+    out = {f"global_{k}": v.detach().float().cpu().numpy() for k, v in model.items()}
+    out.update({k: np.atleast_1d(np.asarray(v, dtype=np.float64)) for k, v in res.items()})
+    for k, a in out.items():
+        if a.size > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            out[k] = a.reshape(-1)[idx]
+    return out
 
 
 class ClockSampler:
@@ -178,11 +208,12 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return t.tolist()
 
-    def measure(eng, drain, want_clocks):
+    def measure(eng, drain, want_clocks, dump=False):
         """W warm-up rounds, then K device-timed rounds (resident inputs), K e2e rounds (pinned
         host inputs in, result out, inside the timed interval) and K back-to-back rounds.
         Every timed round: CUDA events on the engine stream, L2 flush + barrier outside the
-        interval, max over ranks."""
+        interval, max over ranks.  ``dump``: also return round_outputs() of the K-th device-timed
+        round (read after it, outside every timed interval)."""
         pool_x = [p.x.reshape(len(p), -1).contiguous().pin_memory() for p in pool]
         ydt = eng.host_y.dtype
         pool_y = [p.y.to(ydt).contiguous().pin_memory() for p in pool]
@@ -225,6 +256,10 @@ def main():
         t_dev = timed(round_only, args.steps)
         errs += drain()
         launches = _launch_count() - launches0
+        outputs = None
+        if dump:
+            sync_all()          # every rank's round, peers' writes into this heap included, has landed
+            outputs = round_outputs(eng)
         t_e2e = timed(round_e2e, args.steps)
         errs += drain()
         sync_all()   # back-to-back (no flush, no per-round barrier) for context
@@ -242,7 +277,7 @@ def main():
         errs += drain()
         return dict(dev_ms=sum(reduce_max(t_dev)), e2e_ms=sum(reduce_max(t_e2e)),
                     pipe_ms=reduce_max([pipelined_ms])[0], launches=int(launches), clocks=clocks,
-                    ledger_errs=errs)
+                    ledger_errs=errs, outputs=outputs)
 
     W = max(args.warmup, 3)
     base = None
@@ -272,7 +307,7 @@ def main():
                                  broadcast=args.broadcast)
     eng.capture()
     drain = (lambda: eng.drain_blocks()) if args.impl == "fused" else (lambda: [])
-    mres = measure(eng, drain, True)
+    mres = measure(eng, drain, True, dump=args.dump_outputs is not None)
     dev_ms, e2e_ms, pipe_ms = mres["dev_ms"], mres["e2e_ms"], mres["pipe_ms"]
     clocks, launches, ledger_errs = mres["clocks"], mres["launches"], mres["ledger_errs"]
 
@@ -322,6 +357,12 @@ def main():
         extra = {"epoch": eng.epoch, "global_loss": eng.global_loss,
                  "graph_captured": bool(getattr(eng, "graphs", None))}
         gl = int(launches)
+
+    if rank == 0 and args.dump_outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in mres["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     if rank == 0:
         K = args.steps

@@ -579,6 +579,10 @@ std::unique_ptr<Ledger> Ledger::restore(const std::string& blob) {
   c.aggregate_count = r.pod<int32_t>(); c.needed_update_count = r.pod<int32_t>();
   c.learning_rate = r.pod<float>(); c.model_size = r.pod<int64_t>();
   c.weight_by_score = r.pod<int32_t>(); c.solo = r.pod<int32_t>(); c.seed = r.pod<uint64_t>();
+  // the constructor zero-fills a model of model_size floats: refuse a size the blob cannot hold
+  // before allocating it (a corrupted size field would otherwise cost gigabytes of host memory)
+  if (c.model_size > static_cast<int64_t>((blob.size() - r.pos) / sizeof(float)))
+    throw std::runtime_error("ledger snapshot: model size mismatch");
   auto LP = std::make_unique<Ledger>(c);
   Ledger& L = *LP;
   L.epoch_ = r.pod<int32_t>();

@@ -279,3 +279,8 @@ def test_device_round_and_snapshot_inputs_are_validated():
     assert ok + bad_n == 300 and bad_n > 0
     with pytest.raises(RuntimeError):
         L.Ledger.restore(blob[: len(blob) // 2])
+    # a model size the blob cannot hold (int64 at byte 28) is refused before the model is allocated
+    huge = bytearray(blob)
+    huge[28:36] = (1 << 40).to_bytes(8, "little")
+    with pytest.raises(RuntimeError, match="model size"):
+        L.Ledger.restore(bytes(huge))

@@ -18,10 +18,14 @@ def test_chrome_trace_and_phase_timer(tmp_path):
     ev = json.load(open(path))["traceEvents"]
     assert [e["name"] for e in ev] == ["train", "round"] and ev[1]["args"] == {"epoch": 1}
     assert all(e["pid"] == 3 and e["dur"] >= 0 for e in ev)
-    t = PhaseTimer()  # no CUDA here: becomes a no-op but keeps the API
+    t = PhaseTimer()  # without CUDA: a no-op that keeps the API
     with t.phase("x"):
         pass
-    assert t.summary() == {} or "x" in t.summary()
+    s = t.summary()   # (resets the timer: read it once)
+    if torch.cuda.is_available():
+        assert s["x"]["count"] == 1 and s["x"]["total_ms"] >= 0
+    else:
+        assert s == {}
 
 
 def test_runlog_prints_reference_lines(tmp_path):
