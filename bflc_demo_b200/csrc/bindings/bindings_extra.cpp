@@ -11,6 +11,7 @@
 #include <optional>
 
 #include "bflc_kernels.h"
+#include "mc_round.h"
 #include "symm_heap.hpp"
 
 namespace py = pybind11;
@@ -139,6 +140,22 @@ void bind_extra(py::module_& m) {
     d["state_global_loss_off"] = offsetof(bflc::RoundState, global_loss);
     d["state_digest_off"] = offsetof(bflc::RoundState, model_digest);
     d["CUtensorMap"] = sizeof(CUtensorMap);
+    // multi-client engine (mc_round.h)
+    d["McState"] = sizeof(bflc::McState);
+    d["McPlan"] = sizeof(bflc::McPlan);
+    d["McBlockRecord"] = sizeof(bflc::McBlockRecord);
+    d["McClients"] = sizeof(bflc::McClients);
+    d["kMcMaxClients"] = bflc::kMcMaxClients;
+    d["mc_plan_is_trainer_off"] = offsetof(bflc::McPlan, is_trainer);
+    d["mc_plan_barrier_off"] = offsetof(bflc::McPlan, barrier);
+    d["mc_plan_opt_step_off"] = offsetof(bflc::McPlan, opt_step);
+    d["mc_plan_loss_sum_off"] = offsetof(bflc::McPlan, loss_sum);
+    d["mc_plan_train_correct_off"] = offsetof(bflc::McPlan, train_correct);
+    d["mc_plan_n_cand_off"] = offsetof(bflc::McPlan, n_cand);
+    d["mc_plan_cand_off"] = offsetof(bflc::McPlan, cand);
+    d["mc_plan_n_comm_off"] = offsetof(bflc::McPlan, n_comm);
+    d["mc_plan_comm_off"] = offsetof(bflc::McPlan, comm);
+    d["mc_plan_correct_off"] = offsetof(bflc::McPlan, correct);
     return d;
   });
 

@@ -1,0 +1,123 @@
+// Bindings of the multi-client engine's kernels (csrc/include/mc_round.h).
+#include <ATen/cuda/CUDAContext.h>
+#include <torch/extension.h>
+
+#include <cstring>
+
+#include "bflc_kernels.h"
+#include "mc_round.h"
+
+namespace py = pybind11;
+
+namespace {
+
+void check(cudaError_t e, const char* what) {
+  TORCH_CHECK(e == cudaSuccess, "bflc::", what, " failed: ", cudaGetErrorString(e));
+}
+cudaStream_t cur_stream() { return at::cuda::getCurrentCUDAStream().stream(); }
+
+template <typename T>
+T* P(int64_t addr) { return reinterpret_cast<T*>(static_cast<uintptr_t>(addr)); }
+
+// {st, plan, ring, ring_slots, clients, global_master, global_shadow, n_params}
+bflc::McArgs make_mc(const py::dict& d) {
+  bflc::McArgs a;
+  std::memset(&a, 0, sizeof(a));
+  a.st = P<bflc::McState>(d["st"].cast<int64_t>());
+  a.plan = P<bflc::McPlan>(d["plan"].cast<int64_t>());
+  a.ring = P<bflc::McBlockRecord>(d["ring"].cast<int64_t>());
+  a.ring_slots = d["ring_slots"].cast<int>();
+  a.clients = P<const bflc::McClients>(d["clients"].cast<int64_t>());
+  a.global_master = P<float>(d["global_master"].cast<int64_t>());
+  a.global_shadow = P<uint16_t>(d["global_shadow"].cast<int64_t>());
+  a.n_params = d["n_params"].cast<int64_t>();
+  TORCH_CHECK(a.st && a.plan && a.ring && a.clients && a.ring_slots > 0, "incomplete multi-client args");
+  return a;
+}
+
+}  // namespace
+
+void bind_mc(py::module_& m) {
+  m.def("mc_state_init_bytes", [](int n_clients, int n_comm, int n_aggregate, int n_needed, int seed,
+                                  uint32_t straggler_mask, std::vector<int> roles) {
+    TORCH_CHECK(n_clients >= 1 && n_clients <= bflc::kMcMaxClients && (int)roles.size() == n_clients,
+                "1 <= clients <= 32, one role per client");
+    bflc::McState st;
+    std::memset(&st, 0, sizeof(st));
+    st.n_clients = n_clients; st.n_comm = n_comm; st.n_aggregate = n_aggregate; st.n_needed = n_needed;
+    st.seed = static_cast<uint32_t>(seed); st.straggler_mask = straggler_mask;
+    for (int r = 0; r < n_clients; ++r) st.role[r] = static_cast<uint32_t>(roles[r]);
+    return py::bytes(reinterpret_cast<const char*>(&st), sizeof(st));
+  });
+  m.def("mc_clients_bytes", [](std::vector<int64_t> master, std::vector<int64_t> shadow, std::vector<int64_t> blob) {
+    TORCH_CHECK(master.size() <= (size_t)bflc::kMcMaxClients && shadow.size() == master.size() &&
+                (blob.empty() || blob.size() == master.size()), "per-client pointer lists");
+    bflc::McClients c;
+    std::memset(&c, 0, sizeof(c));
+    for (size_t i = 0; i < master.size(); ++i) {
+      c.master[i] = P<float>(master[i]);
+      c.shadow[i] = P<uint16_t>(shadow[i]);
+      c.blob[i] = blob.empty() ? nullptr : P<uint8_t>(blob[i]);
+    }
+    return py::bytes(reinterpret_cast<const char*>(&c), sizeof(c));
+  });
+  m.def("mc_plan_round", [](const py::dict& d, int steps) {
+    check(bflc::mc_plan_round(make_mc(d), steps, cur_stream()), "mc_plan_round");
+  });
+  m.def("mc_byzantine", [](const py::dict& d, std::vector<int> ids, double scale) {
+    check(bflc::mc_byzantine(make_mc(d), ids.data(), (int)ids.size(), (float)scale, cur_stream()), "mc_byzantine");
+  });
+  m.def("mc_consensus", [](const py::dict& d, int n_val, int n_samples, int n_loss_terms, bool weight_by_score) {
+    check(bflc::mc_consensus(make_mc(d), n_val, n_samples, n_loss_terms, weight_by_score ? 1 : 0, cur_stream()),
+          "mc_consensus");
+  });
+  m.def("mc_fedavg", [](const py::dict& d, int n_clients) {
+    check(bflc::mc_fedavg(make_mc(d), n_clients, cur_stream()), "mc_fedavg");
+  });
+  m.def("mc_broadcast_blob", [](const py::dict& d, at::Tensor src, int n_clients) {
+    check(bflc::mc_broadcast_blob(make_mc(d), src.data_ptr<uint8_t>(), src.numel(), n_clients, cur_stream()),
+          "mc_broadcast_blob");
+  });
+  m.def("mc_val", [](int64_t plan_ptr, int64_t correct_ptr, at::Tensor x_maps, at::Tensor w_maps,
+                     int64_t clients_ptr, int64_t b1_off, int64_t b2_off, at::Tensor labels,
+                     int64_t labels_stride, int n_val, int in_dim, int hidden, int n_classes, int max_cand,
+                     int max_comm, const std::optional<at::Tensor>& x_sf, int64_t x_sf_stride) {
+    bflc::McValArgs r;
+    r.n_val = n_val; r.in_dim = in_dim; r.hidden = hidden; r.n_classes = n_classes;
+    r.max_cand = max_cand; r.max_comm = max_comm;
+    r.plan = P<const bflc::McPlan>(plan_ptr);
+    r.correct = P<unsigned int>(correct_ptr);
+    r.x_maps = reinterpret_cast<const CUtensorMap*>(x_maps.data_ptr());
+    r.w_maps = reinterpret_cast<const CUtensorMap*>(w_maps.data_ptr());
+    r.clients = P<const bflc::McClients>(clients_ptr);
+    r.b1_off = b1_off; r.b2_off = b2_off;
+    r.labels = labels.data_ptr<int32_t>(); r.labels_stride = labels_stride;
+    if (x_sf.has_value()) {
+      r.fp8 = true;
+      r.x_sf = x_sf->data_ptr<uint8_t>(); r.x_sf_stride = x_sf_stride;
+    }
+    check(bflc::mc_val_sm100(r, cur_stream()), "mc_val_sm100");
+  }, py::arg("plan_ptr"), py::arg("correct_ptr"), py::arg("x_maps"), py::arg("w_maps"), py::arg("clients_ptr"),
+     py::arg("b1_off"), py::arg("b2_off"), py::arg("labels"), py::arg("labels_stride"), py::arg("n_val"),
+     py::arg("in_dim"), py::arg("hidden"), py::arg("n_classes"), py::arg("max_cand"), py::arg("max_comm"),
+     py::arg("x_sf") = py::none(), py::arg("x_sf_stride") = 0);
+  // TMA descriptor of a K-major operand [rows][K] (row pitch ld elements), box rows_tile x 128 B
+  m.def("operand_map", [](int64_t ptr, int64_t ld, int rows, int K, bool fp8, int rows_tile) {
+    CUtensorMap t;
+    bflc::GemmOperand op{P<const void>(ptr), ld, 0, false};
+    check(bflc::gemm_make_operand_map(&t, op, fp8 ? bflc::DType::FP8_E4M3 : bflc::DType::BF16, rows, K, 1, rows_tile),
+          "gemm_make_operand_map");
+    return py::bytes(reinterpret_cast<const char*>(&t), sizeof(t));
+  });
+  // a GemmDynamic record (device-resident per-launch GEMM / mlp_val arguments) built on the host
+  m.def("gemm_dynamic_bytes", [](int active, std::vector<int> map_index, std::vector<int64_t> bias) {
+    TORCH_CHECK(map_index.size() <= (size_t)bflc::kMaxRanks && bias.size() <= (size_t)bflc::kMaxRanks,
+                "at most kMaxRanks batches");
+    bflc::GemmDynamic g;
+    std::memset(&g, 0, sizeof(g));
+    g.active_batches = active;
+    for (size_t i = 0; i < map_index.size(); ++i) g.map_index[i] = map_index[i];
+    for (size_t i = 0; i < bias.size(); ++i) g.bias[i] = P<const float>(bias[i]);
+    return py::bytes(reinterpret_cast<const char*>(&g), sizeof(g));
+  });
+}

@@ -99,6 +99,7 @@ py::bytes gemm_b_map(int64_t ptr, int64_t N, int64_t K, int64_t ldb, bool b_mn, 
 
 void bind_extra(py::module_& m);  // defined in bindings_extra.cpp
 void bind_nn(py::module_& m);     // defined in bindings_nn.cpp
+void bind_mc(py::module_& m);     // defined in bindings_mc.cpp
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.doc() = "bflc_demo_b200 native kernels (sm_100a)";
@@ -136,4 +137,5 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("launch_count", [] { return bflc::launch_count(); });
   bind_extra(m);
   bind_nn(m);
+  bind_mc(m);
 }

@@ -22,6 +22,7 @@
 #include "bflc_kernels.h"
 #include "epi_common.cuh"
 #include "launch.cuh"
+#include "mc_round.h"
 #include "sm100_ptx.cuh"
 
 namespace bflc {
@@ -71,100 +72,100 @@ __device__ __forceinline__ void val_stamp(unsigned long long* stamps, int slot) 
   atomicMax(stamps + slot, t);
 }
 
-template <bool FP8>
-__global__ void __launch_bounds__(kThreads, 1)
-mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>(
-      (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-  uint8_t* sf_smem = smem + kOffSf;
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + kOffBar);
-  uint64_t* empty = full + kCStages;
-  uint64_t* w2k = empty + kCStages;
-  uint64_t* acc_h = w2k + 1;
-  uint64_t* h_ready = acc_h + 1;
-  uint64_t* acc_l = h_ready + 1;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_l + 1);
-  float* sb = reinterpret_cast<float*>(smem + kOffBar + kBarBytes);
+// Shared-memory carve-up of one validation CTA (both kernels below).
+struct ValSmem {
+  uint8_t* smem; uint8_t* sf_smem;
+  uint64_t* full; uint64_t* empty; uint64_t* w2k; uint64_t* acc_h; uint64_t* h_ready; uint64_t* acc_l;
+  uint32_t* tmem_slot; float* sb;
+};
 
-  ptx::pdl_launch_dependents();
+__device__ __forceinline__ ValSmem val_smem(uint8_t* smem_raw) {
+  ValSmem s;
+  s.smem = reinterpret_cast<uint8_t*>(
+      (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
+  s.sf_smem = s.smem + kOffSf;
+  s.full = reinterpret_cast<uint64_t*>(s.smem + kOffBar);
+  s.empty = s.full + kCStages;
+  s.w2k = s.empty + kCStages;
+  s.acc_h = s.w2k + 1;
+  s.h_ready = s.acc_h + 1;
+  s.acc_l = s.h_ready + 1;
+  s.tmem_slot = reinterpret_cast<uint32_t*>(s.acc_l + 1);
+  s.sb = reinterpret_cast<float*>(s.smem + kOffBar + kBarBytes);
+  return s;
+}
+
+// mbarrier init + TMEM allocation (before griddepcontrol.wait); returns the TMEM base
+__device__ __forceinline__ uint32_t val_setup(const ValSmem& S, const CUtensorMap* prefetch) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int z = blockIdx.y, m0 = blockIdx.x * kBM;
   if (warp == 0 && lane == 0) {
-    ptx::tma_prefetch_desc(&tmX);
+    if (prefetch != nullptr) ptx::tma_prefetch_desc(prefetch);
     for (int s = 0; s < kCStages; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
+      ptx::mbar_init(&S.full[s], 1);
+      ptx::mbar_init(&S.empty[s], 1);
     }
-    ptx::mbar_init(w2k, 1); ptx::mbar_init(acc_h, 1); ptx::mbar_init(acc_l, 1);
-    ptx::mbar_init(h_ready, kEpiWarps * 32);
+    ptx::mbar_init(S.w2k, 1); ptx::mbar_init(S.acc_h, 1); ptx::mbar_init(S.acc_l, 1);
+    ptx::mbar_init(S.h_ready, kEpiWarps * 32);
     ptx::fence_mbar_init();
   }
-  if (warp == 1) ptx::tmem_alloc(tmem_slot, kTmemCols);
+  if (warp == 1) ptx::tmem_alloc(S.tmem_slot, kTmemCols);
   ptx::tc_fence_before_sync();
   __syncthreads();
   ptx::tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-  ptx::pdl_wait();
-  const bool inactive = (v.pred != nullptr && *v.pred == 0) || z >= v.dyn1->active_batches;
-  if (inactive) {
-    if (warp == 1) ptx::tmem_dealloc(tmem_base, kTmemCols);
-    return;
+  return *S.tmem_slot;
+}
+
+__device__ __forceinline__ void val_teardown(uint32_t tmem_base) {
+  __syncthreads();
+  if ((threadIdx.x >> 5) == 1) {
+    ptx::tc_fence_after_sync();
+    ptx::tmem_dealloc(tmem_base, kTmemCols);
   }
-  const int kb_d = FP8 ? v.ql.kb1 : (v.in_dim + 63) / 64;
+}
+
+// What one CTA validates: 128 rows of x (map tx, row m0) against one candidate.
+struct ChainJob {
+  const CUtensorMap* tx; const CUtensorMap* m1; const CUtensorMap* m2;
+  const float* b1; const float* b2;   // bf16 candidate biases (fp8: inside the blob)
+  const uint8_t* blob;                // fp8 candidate (Mx8MlpLayout)
+  const uint8_t* x_sf;                // fp8: scale chunks of x
+  const int32_t* labels; unsigned int* correct;
+  const uint32_t* wait_flag; uint32_t wait_value;   // optional: wait until *wait_flag >= wait_value
+};
+
+// The chain fwd1 -> relu -> fwd2 -> argmax == label of one (128 rows, candidate) tile, warp
+// specialised: warp 0 TMA producer, warp 1 MMA issuer, warps 2..9 epilogue.
+template <bool FP8>
+__device__ __forceinline__ void val_chain(const ValSmem& S, uint32_t tmem_base, const ChainJob& j, int m0,
+                                          int n_val, int in_dim, int n_classes, const Mx8MlpLayout& ql) {
+  uint8_t* smem = S.smem;
+  uint8_t* sf_smem = S.sf_smem;
+  uint64_t* full = S.full;
+  uint64_t* empty = S.empty;
+  uint64_t* w2k = S.w2k;
+  uint64_t* acc_h = S.acc_h;
+  uint64_t* h_ready = S.h_ready;
+  uint64_t* acc_l = S.acc_l;
+  float* sb = S.sb;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int kb_d = FP8 ? ql.kb1 : (in_dim + 63) / 64;
   const uint32_t hi = (1024u >> 4) | (1u << 14) | (2u << 29);
   const uint32_t base_lo = ptx::smem_u32(smem) >> 4;
-  const uint8_t* blob = FP8 ? v.cand_blob[z] : nullptr;
-
-  if (FP8 && v.cand_src != nullptr) {
-    // ---- fused gather (reference: QueryAllUpdates, CommitteePrecompiled.cpp:299-311).  The
-    // gridDim.x CTAs that validate candidate z each copy 1/gridDim.x of z's blob out of the
-    // trainer's HBM with 16-byte P2P loads as soon as its FLAG_TRAINED is up, publish their share
-    // (device-scope fence + counter), wait for the others' shares and only then start the TMA /
-    // bulk loads of the local copy.  Every candidate crosses NVLink once per committee rank, and
-    // there is no pull kernel in front of the validation.
-    if (threadIdx.x == 0 && v.stamps != nullptr && blockIdx.x == 0 && z == 0) val_stamp(v.stamps, STAMP_PULL_BEGIN);
-    if (threadIdx.x == 0 && v.dyn1->wait_flag[z] != nullptr)
-      ptx::wait_flag_ge(v.dyn1->wait_flag[z], v.dyn1->wait_value);
-    __syncthreads();
-    const float4* src = reinterpret_cast<const float4*>(v.cand_src[z]);
-    float4* dst = reinterpret_cast<float4*>(const_cast<uint8_t*>(blob));
-    const long long n16 = v.blob_bytes >> 4;
-    const long long per = (n16 + gridDim.x - 1) / gridDim.x;
-    const long long lo = per * blockIdx.x, hi = lo + per < n16 ? lo + per : n16;
-    for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) dst[i] = ptx::ld_peer_f4(src + i);
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      atomicAdd(v.pull_cnt + z, 1u);
-      unsigned long long spins = 0;
-      unsigned int have;
-      do {
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(have) : "l"(v.pull_cnt + z) : "memory");
-        if (have >= gridDim.x) break;
-        __nanosleep(20);
-      } while (++spins < (1ull << 26));
-      if (have < gridDim.x) __trap();   // a sibling CTA never arrived: co-residency assumption broken
-      if (v.stamps != nullptr && blockIdx.x == 0) val_stamp(v.stamps, STAMP_PULL_END);
-    }
-    __syncthreads();
-    ptx::fence_proxy_async_all();   // the others' generic-proxy stores -> this CTA's TMA / bulk loads
-  }
 
   if (warp == 0) {
-    if (v.dyn1->wait_flag[z] != nullptr) {   // candidate z's trainer has published its upload
-      if (lane == 0) ptx::wait_flag_ge(v.dyn1->wait_flag[z], v.dyn1->wait_value);
+    if (j.wait_flag != nullptr) {   // candidate z's trainer has published its upload
+      if (lane == 0) ptx::wait_flag_ge(j.wait_flag, j.wait_value);
       __syncwarp();
     }
-    const CUtensorMap* m1 = v.maps + v.dyn1->map_index[z];
-    const CUtensorMap* m2 = v.maps + v.dyn2->map_index[z];
+    const CUtensorMap* m1 = j.m1;
+    const CUtensorMap* m2 = j.m2;
     if (ptx::elect_one()) {
       if (FP8) {
         ptx::mbar_expect_tx(w2k, 2 * 8192 + 2 * kSfChunk);
 #pragma unroll
         for (int kb = 0; kb < 2; ++kb) {
           ptx::tma_load_3d(smem + kOffW2K + kb * 8192, m2, w2k, kb * 128, 0, 0);
-          epi::bulk_g2s(sf_smem + kSfW2 + kb * kSfChunk, blob + v.ql.w2sf + kb * kSfChunk, kSfChunk, w2k);
+          epi::bulk_g2s(sf_smem + kSfW2 + kb * kSfChunk, j.blob + ql.w2sf + kb * kSfChunk, kSfChunk, w2k);
         }
       } else {
         ptx::mbar_expect_tx(w2k, 32768);
@@ -182,16 +183,16 @@ mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
         if (FP8) {
           uint8_t* sf = sf_smem + s * kSfStage;
           ptx::mbar_expect_tx(&full[s], kCStage + kSfStage);
-          ptx::tma_load_3d(sa, &tmX, &full[s], i * 128, m0, 0);
+          ptx::tma_load_3d(sa, j.tx, &full[s], i * 128, m0, 0);
           ptx::tma_load_3d(sa + kCA, m1, &full[s], i * 128, 0, 0);
-          epi::bulk_g2s(sf, v.x_sf + (static_cast<long long>(m0 >> 7) * kb_d + i) * kSfChunk, kSfChunk, &full[s]);
+          epi::bulk_g2s(sf, j.x_sf + (static_cast<long long>(m0 >> 7) * kb_d + i) * kSfChunk, kSfChunk, &full[s]);
           // W1: 256 rows = two 128-row blocks of scale chunks
-          epi::bulk_g2s(sf + kSfChunk, blob + v.ql.w1sf + static_cast<long long>(i) * kSfChunk, kSfChunk, &full[s]);
-          epi::bulk_g2s(sf + 2 * kSfChunk, blob + v.ql.w1sf + (static_cast<long long>(kb_d) + i) * kSfChunk, kSfChunk,
+          epi::bulk_g2s(sf + kSfChunk, j.blob + ql.w1sf + static_cast<long long>(i) * kSfChunk, kSfChunk, &full[s]);
+          epi::bulk_g2s(sf + 2 * kSfChunk, j.blob + ql.w1sf + (static_cast<long long>(kb_d) + i) * kSfChunk, kSfChunk,
                         &full[s]);
         } else {
           ptx::mbar_expect_tx(&full[s], kCStage);
-          ptx::tma_load_3d(sa, &tmX, &full[s], i * 64, m0, 0);
+          ptx::tma_load_3d(sa, j.tx, &full[s], i * 64, m0, 0);
           ptx::tma_load_3d(sa + kCA, m1, &full[s], i * 64, 0, 0);
         }
       }
@@ -265,12 +266,12 @@ mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
   } else {
     // warps 2..9: q = TMEM lane quarter, half = which four 32-column chunks of h this warp converts
     const int q = warp & 3, half = (warp - 2) >> 2, rl = q * 32 + lane, row = m0 + rl;
-    const bool row_ok = row < v.n_val;
-    const int C = v.n_classes;
+    const bool row_ok = row < n_val;
+    const int C = n_classes;
     {
       const int et = threadIdx.x - 64;
-      const float* b1 = FP8 ? reinterpret_cast<const float*>(blob + v.ql.b1) : v.dyn1->bias[z];
-      const float* b2 = FP8 ? reinterpret_cast<const float*>(blob + v.ql.b2) : v.dyn2->bias[z];
+      const float* b1 = FP8 ? reinterpret_cast<const float*>(j.blob + ql.b1) : j.b1;
+      const float* b2 = FP8 ? reinterpret_cast<const float*>(j.blob + ql.b2) : j.b2;
       sb[et] = b1 != nullptr ? b1[et] : 0.f;            // kEpiWarps * 32 == kChainH
       if (et < 64) sb[kChainH + et] = (b2 != nullptr && et < C) ? b2[et] : 0.f;
       asm volatile("bar.sync 1, 256;" ::: "memory");
@@ -313,7 +314,7 @@ mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
     if (half == 0) {     // the 64 logits of a row: one thread
     ptx::mbar_wait(acc_l, 0);
     ptx::tc_fence_after_sync();
-    const int32_t label = row_ok ? v.labels[row] : -1;
+    const int32_t label = row_ok ? j.labels[row] : -1;
     float vmax = -INFINITY;
     int amax = -1;
 #pragma unroll
@@ -329,15 +330,119 @@ mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
       }
     }
     const unsigned cnt = __popc(__ballot_sync(0xffffffffu, row_ok && amax == label));
-    if (lane == 0 && cnt) atomicAdd(v.correct + z, cnt);
+    if (lane == 0 && cnt) atomicAdd(j.correct, cnt);
     }
     ptx::tc_fence_before_sync();
   }
-  __syncthreads();
-  if (warp == 1) {
-    ptx::tc_fence_after_sync();
-    ptx::tmem_dealloc(tmem_base, kTmemCols);
+}
+
+template <bool FP8>
+__global__ void __launch_bounds__(kThreads, 1)
+mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
+  extern __shared__ uint8_t smem_raw[];
+  const ValSmem S = val_smem(smem_raw);
+  ptx::pdl_launch_dependents();
+  const int warp = threadIdx.x >> 5;
+  const int z = blockIdx.y, m0 = blockIdx.x * kBM;
+  const uint32_t tmem_base = val_setup(S, &tmX);
+  ptx::pdl_wait();
+  const bool inactive = (v.pred != nullptr && *v.pred == 0) || z >= v.dyn1->active_batches;
+  if (inactive) {
+    if (warp == 1) ptx::tmem_dealloc(tmem_base, kTmemCols);
+    return;
   }
+  const uint8_t* blob = FP8 ? v.cand_blob[z] : nullptr;
+
+  if (FP8 && v.cand_src != nullptr) {
+    // ---- fused gather (reference: QueryAllUpdates, CommitteePrecompiled.cpp:299-311).  The
+    // gridDim.x CTAs that validate candidate z each copy 1/gridDim.x of z's blob out of the
+    // trainer's HBM with 16-byte P2P loads as soon as its FLAG_TRAINED is up, publish their share
+    // (device-scope fence + counter), wait for the others' shares and only then start the TMA /
+    // bulk loads of the local copy.  Every candidate crosses NVLink once per committee rank, and
+    // there is no pull kernel in front of the validation.
+    if (threadIdx.x == 0 && v.stamps != nullptr && blockIdx.x == 0 && z == 0) val_stamp(v.stamps, STAMP_PULL_BEGIN);
+    if (threadIdx.x == 0 && v.dyn1->wait_flag[z] != nullptr)
+      ptx::wait_flag_ge(v.dyn1->wait_flag[z], v.dyn1->wait_value);
+    __syncthreads();
+    const float4* src = reinterpret_cast<const float4*>(v.cand_src[z]);
+    float4* dst = reinterpret_cast<float4*>(const_cast<uint8_t*>(blob));
+    const long long n16 = v.blob_bytes >> 4;
+    const long long per = (n16 + gridDim.x - 1) / gridDim.x;
+    const long long lo = per * blockIdx.x, hi = lo + per < n16 ? lo + per : n16;
+    for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) dst[i] = ptx::ld_peer_f4(src + i);
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      atomicAdd(v.pull_cnt + z, 1u);
+      unsigned long long spins = 0;
+      unsigned int have;
+      do {
+        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(have) : "l"(v.pull_cnt + z) : "memory");
+        if (have >= gridDim.x) break;
+        __nanosleep(20);
+      } while (++spins < (1ull << 26));
+      if (have < gridDim.x) __trap();   // a sibling CTA never arrived: co-residency assumption broken
+      if (v.stamps != nullptr && blockIdx.x == 0) val_stamp(v.stamps, STAMP_PULL_END);
+    }
+    __syncthreads();
+    ptx::fence_proxy_async_all();   // the others' generic-proxy stores -> this CTA's TMA / bulk loads
+  }
+
+  ChainJob j;
+  j.tx = &tmX;
+  j.m1 = v.maps + v.dyn1->map_index[z];
+  j.m2 = v.maps + v.dyn2->map_index[z];
+  j.b1 = FP8 ? nullptr : v.dyn1->bias[z];
+  j.b2 = FP8 ? nullptr : v.dyn2->bias[z];
+  j.blob = blob; j.x_sf = v.x_sf;
+  j.labels = v.labels; j.correct = v.correct + z;
+  j.wait_flag = v.dyn1->wait_flag[z]; j.wait_value = v.dyn1->wait_value;
+  val_chain<FP8>(S, tmem_base, j, m0, v.n_val, v.in_dim, v.n_classes, v.ql);
+  val_teardown(tmem_base);
+}
+
+// Multi-client committee validation (engine/multiclient.py): CTA (m-tile, candidate slot z,
+// committee slot k).  Who is candidate z and member k comes from the round plan; the candidate is
+// read in place from its client's buffers (bf16 work shadow + fp32 biases, or the fp8 blob), the
+// rows are the first n_val rows of the member's own shard.
+struct McVal {
+  int n_val, in_dim, n_classes;
+  const McPlan* plan; unsigned int* correct;
+  const CUtensorMap* x_maps; const CUtensorMap* w_maps;
+  const McClients* clients; long long b1_off, b2_off;
+  const int32_t* labels; long long labels_stride;
+  const uint8_t* x_sf; long long x_sf_stride;
+  Mx8MlpLayout ql;
+};
+
+template <bool FP8>
+__global__ void __launch_bounds__(kThreads, 1)
+mc_val_kernel(const McVal v) {
+  extern __shared__ uint8_t smem_raw[];
+  const ValSmem S = val_smem(smem_raw);
+  ptx::pdl_launch_dependents();
+  const int warp = threadIdx.x >> 5;
+  const int z = blockIdx.y, k = blockIdx.z, m0 = blockIdx.x * kBM;
+  const uint32_t tmem_base = val_setup(S, nullptr);
+  ptx::pdl_wait();
+  if (z >= v.plan->n_cand || k >= v.plan->n_comm) {
+    if (warp == 1) ptx::tmem_dealloc(tmem_base, kTmemCols);
+    return;
+  }
+  const int member = v.plan->comm[k], cand = v.plan->cand[z];
+  ChainJob j;
+  j.tx = v.x_maps + member;
+  j.m1 = v.w_maps + cand;
+  j.m2 = v.w_maps + kMcMaxClients + cand;
+  j.b1 = FP8 ? nullptr : v.clients->master[cand] + v.b1_off;
+  j.b2 = FP8 ? nullptr : v.clients->master[cand] + v.b2_off;
+  j.blob = FP8 ? v.clients->blob[cand] : nullptr;
+  j.x_sf = FP8 ? v.x_sf + member * v.x_sf_stride : nullptr;
+  j.labels = v.labels + member * v.labels_stride;
+  j.correct = v.correct + member * kMcMaxClients + cand;
+  j.wait_flag = nullptr; j.wait_value = 0u;
+  val_chain<FP8>(S, tmem_base, j, m0, v.n_val, v.in_dim, v.n_classes, v.ql);
+  val_teardown(tmem_base);
 }
 
 }  // namespace
@@ -376,6 +481,35 @@ cudaError_t mlp_val_sm100(const MlpValArgs& r, cudaStream_t stream) {
   const dim3 grid((r.n_val + kBM - 1) / kBM, r.max_cand);
   if (r.fp8) return launch_pdl(mlp_val_kernel<true>, grid, dim3(kThreads), kValSmem, stream, tx, v);
   return launch_pdl(mlp_val_kernel<false>, grid, dim3(kThreads), kValSmem, stream, tx, v);
+}
+
+cudaError_t mc_val_sm100(const McValArgs& r, cudaStream_t stream) {
+  bind_context_once();
+  if (r.hidden != kChainH || r.n_classes > 64 || r.in_dim % 8 || r.n_val <= 0 || r.max_cand <= 0 ||
+      r.max_cand > kMcMaxClients || r.max_comm <= 0 || r.max_comm > kMcMaxClients || r.plan == nullptr ||
+      r.correct == nullptr || r.x_maps == nullptr || r.w_maps == nullptr || r.clients == nullptr ||
+      r.labels == nullptr)
+    return cudaErrorInvalidValue;
+  if (r.fp8 && (r.x_sf == nullptr || r.in_dim % 16)) return cudaErrorInvalidValue;
+  McVal v{};
+  v.n_val = r.n_val; v.in_dim = r.in_dim; v.n_classes = r.n_classes;
+  v.plan = r.plan; v.correct = r.correct; v.x_maps = r.x_maps; v.w_maps = r.w_maps;
+  v.clients = r.clients; v.b1_off = r.b1_off; v.b2_off = r.b2_off;
+  v.labels = r.labels; v.labels_stride = r.labels_stride;
+  v.x_sf = r.x_sf; v.x_sf_stride = r.x_sf_stride;
+  v.ql = mx8_mlp_layout(r.in_dim, r.hidden);
+  static bool configured[2] = {false, false};
+  cudaError_t e;
+  if (!configured[r.fp8 ? 1 : 0]) {
+    e = r.fp8 ? cudaFuncSetAttribute(mc_val_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kValSmem)
+              : cudaFuncSetAttribute(mc_val_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kValSmem);
+    if (e != cudaSuccess) return e;
+    configured[r.fp8 ? 1 : 0] = true;
+  }
+  note_launch();
+  const dim3 grid((r.n_val + kBM - 1) / kBM, r.max_cand, r.max_comm);
+  if (r.fp8) return launch_pdl(mc_val_kernel<true>, grid, dim3(kThreads), kValSmem, stream, v);
+  return launch_pdl(mc_val_kernel<false>, grid, dim3(kThreads), kValSmem, stream, v);
 }
 
 }  // namespace bflc

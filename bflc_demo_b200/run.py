@@ -2,6 +2,7 @@
 reference, python-sdk/main.py:343-358, for one NVSwitch box):
 
     python -m bflc_demo_b200.run --model mlp --rounds 20                       # 1 GPU, solo
+    python -m bflc_demo_b200.run --clients 20 --rounds 20     # 20 clients on 1 GPU (20/4/10/6)
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 \\
         -m bflc_demo_b200.run --model resnet18 --rounds 5 --byzantine 7       # config #4
 
@@ -42,6 +43,12 @@ def main(argv=None):
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp8"],
                     help="fp8: block-scaled (MXFP8) forward GEMMs (the MLP keeps the fused persistent trainer)")
     ap.add_argument("--generic", action="store_true", help="run the MLP through GenericFedEngine")
+    ap.add_argument("--clients", type=int, default=0,
+                    help="clients (default: one per GPU); more than WORLD_SIZE on one GPU runs the "
+                         "MLP through MultiClientEngine")
+    ap.add_argument("--committee", type=int, default=4, help="--clients: committee size (COMM_COUNT)")
+    ap.add_argument("--needed", type=int, default=10, help="--clients: NEEDED_UPDATE_COUNT")
+    ap.add_argument("--aggregate", type=int, default=6, help="--clients: AGGREGATE_COUNT")
     a = ap.parse_args(argv)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -50,6 +57,12 @@ def main(argv=None):
     torch.cuda.set_device(lr_)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", lr_))
+
+    if a.clients > world:
+        if world > 1:
+            raise SystemExit(f"--clients {a.clients} > WORLD_SIZE {world}: several clients per GPU is "
+                             "supported on a single GPU only")
+        return run_multiclient(a)
 
     defaults = dict(mlp=(4096, 512, 0.05), lenet5=(2048, 128, 0.05), resnet18=(512, 64, 0.02),
                     bert=(64, 16, 0.002))[a.model]
@@ -103,6 +116,36 @@ def main(argv=None):
         torch.cuda.synchronize()
         dist.barrier()
         dist.destroy_process_group()
+
+
+def run_multiclient(a):
+    """--clients N on one GPU: N virtual clients, the committee protocol in one captured graph."""
+    from .engine.multiclient import MultiClientEngine
+    if a.model != "mlp":
+        raise SystemExit("--clients runs the MLP only")
+    S, B, LR = a.samples or 4096, a.batch or 512, a.lr or (0.002 if a.optimizer == "adam" else 0.05)
+    cfg = FLConfig(clients=a.clients, committee_size=a.committee, needed_updates=a.needed,
+                   aggregate_count=a.aggregate, batch_size=B, samples_per_client=S, learning_rate=LR,
+                   optimizer=a.optimizer, byzantine_ranks=a.byzantine, ring_slots=1024,
+                   dtype=a.dtype).validate()
+    shards = femnist_like(a.clients, S, seed=7)
+    test = femnist_like(1, 2048, seed=7, only=0)[0]
+    eng = MultiClientEngine(cfg, shards, device=0)
+    eng.capture()
+    log = RunLog(rank=0)
+    timer = PhaseTimer()
+    t0 = time.time()
+    for _ in range(a.rounds):
+        with timer.phase("round"):
+            eng.run_round()
+        st = eng.read_state()
+        log.round(st["epoch"] - 1, st["global_loss"], test_acc=eng.evaluate(test),
+                  committee=[r for r, x in enumerate(st["roles"]) if x & 2])
+    errs = eng.drain_blocks()
+    summary = dict(rounds=a.rounds, clients=a.clients, wall_s=round(time.time() - t0, 3),
+                   timing=timer.summary(), ledger_mismatches=errs, chain_ok=eng.host_ledger.verify_chain(),
+                   blocks=eng.host_ledger.n_blocks(), launches_per_round=eng.launches_per_round)
+    print("SUMMARY " + json.dumps(summary))
 
 
 if __name__ == "__main__":
