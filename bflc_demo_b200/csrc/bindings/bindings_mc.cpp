@@ -2,6 +2,7 @@
 #include <ATen/cuda/CUDAContext.h>
 #include <torch/extension.h>
 
+#include <cstdint>
 #include <cstring>
 
 #include "bflc_kernels.h"
@@ -49,27 +50,45 @@ void bind_mc(py::module_& m) {
     for (int r = 0; r < n_clients; ++r) st.role[r] = static_cast<uint32_t>(roles[r]);
     return py::bytes(reinterpret_cast<const char*>(&st), sizeof(st));
   });
-  m.def("mc_clients_bytes", [](std::vector<int64_t> master, std::vector<int64_t> shadow, std::vector<int64_t> blob) {
-    TORCH_CHECK(master.size() <= (size_t)bflc::kMcMaxClients && shadow.size() == master.size() &&
-                (blob.empty() || blob.size() == master.size()), "per-client pointer lists");
+  // per-client lists, one entry per client (blob / x_sf: empty in bf16)
+  m.def("mc_clients_bytes", [](std::vector<int64_t> master, std::vector<int64_t> shadow, std::vector<int64_t> blob,
+                               std::vector<int64_t> labels, std::vector<int64_t> x_sf,
+                               std::vector<int64_t> n_samples, std::vector<int> steps, std::vector<int> n_val,
+                               int batch) {
+    const size_t n = master.size();
+    TORCH_CHECK(n >= 1 && n <= (size_t)bflc::kMcMaxClients, "1 <= clients <= ", bflc::kMcMaxClients);
+    TORCH_CHECK(shadow.size() == n && labels.size() == n && n_samples.size() == n && steps.size() == n &&
+                n_val.size() == n && (blob.empty() || blob.size() == n) && (x_sf.empty() || x_sf.size() == n),
+                "per-client lists: one entry per client");
+    TORCH_CHECK(blob.empty() == x_sf.empty(), "fp8 needs both the blobs and the scale chunks");
+    TORCH_CHECK(batch > 0, "batch must be positive");
     bflc::McClients c;
     std::memset(&c, 0, sizeof(c));
-    for (size_t i = 0; i < master.size(); ++i) {
+    for (size_t i = 0; i < n; ++i) {
+      TORCH_CHECK(steps[i] > 0 && n_val[i] > 0 && n_samples[i] > 0 && n_samples[i] <= 0xffffffffll &&
+                  (int64_t)steps[i] * batch <= (int64_t)INT32_MAX,
+                  "client ", i, ": steps, n_val and n_samples must be positive");
+      TORCH_CHECK(master[i] && shadow[i] && labels[i], "client ", i, ": null pointer");
       c.master[i] = P<float>(master[i]);
       c.shadow[i] = P<uint16_t>(shadow[i]);
       c.blob[i] = blob.empty() ? nullptr : P<uint8_t>(blob[i]);
+      c.labels[i] = P<const int32_t>(labels[i]);
+      c.x_sf[i] = x_sf.empty() ? nullptr : P<const uint8_t>(x_sf[i]);
+      c.n_samples[i] = static_cast<uint32_t>(n_samples[i]);
+      c.steps[i] = steps[i];
+      c.n_val[i] = n_val[i];
     }
+    c.batch = batch;
     return py::bytes(reinterpret_cast<const char*>(&c), sizeof(c));
   });
-  m.def("mc_plan_round", [](const py::dict& d, int steps) {
-    check(bflc::mc_plan_round(make_mc(d), steps, cur_stream()), "mc_plan_round");
+  m.def("mc_plan_round", [](const py::dict& d) {
+    check(bflc::mc_plan_round(make_mc(d), cur_stream()), "mc_plan_round");
   });
   m.def("mc_byzantine", [](const py::dict& d, std::vector<int> ids, double scale) {
     check(bflc::mc_byzantine(make_mc(d), ids.data(), (int)ids.size(), (float)scale, cur_stream()), "mc_byzantine");
   });
-  m.def("mc_consensus", [](const py::dict& d, int n_val, int n_samples, int n_loss_terms, bool weight_by_score) {
-    check(bflc::mc_consensus(make_mc(d), n_val, n_samples, n_loss_terms, weight_by_score ? 1 : 0, cur_stream()),
-          "mc_consensus");
+  m.def("mc_consensus", [](const py::dict& d, bool weight_by_score) {
+    check(bflc::mc_consensus(make_mc(d), weight_by_score ? 1 : 0, cur_stream()), "mc_consensus");
   });
   m.def("mc_fedavg", [](const py::dict& d, int n_clients) {
     check(bflc::mc_fedavg(make_mc(d), n_clients, cur_stream()), "mc_fedavg");
@@ -78,12 +97,19 @@ void bind_mc(py::module_& m) {
     check(bflc::mc_broadcast_blob(make_mc(d), src.data_ptr<uint8_t>(), src.numel(), n_clients, cur_stream()),
           "mc_broadcast_blob");
   });
+  // labels, n_val and (fp8) scale chunks of every member come from its McClients entry
   m.def("mc_val", [](int64_t plan_ptr, int64_t correct_ptr, at::Tensor x_maps, at::Tensor w_maps,
-                     int64_t clients_ptr, int64_t b1_off, int64_t b2_off, at::Tensor labels,
-                     int64_t labels_stride, int n_val, int in_dim, int hidden, int n_classes, int max_cand,
-                     int max_comm, const std::optional<at::Tensor>& x_sf, int64_t x_sf_stride) {
+                     int64_t clients_ptr, int64_t b1_off, int64_t b2_off, int max_n_val, int in_dim, int hidden,
+                     int n_classes, int max_cand, int max_comm, bool fp8) {
+    const int64_t ctm = static_cast<int64_t>(sizeof(CUtensorMap));
+    TORCH_CHECK(max_cand >= 1 && max_cand <= bflc::kMcMaxClients && max_comm >= 1 &&
+                max_comm <= bflc::kMcMaxClients, "1 <= max_cand, max_comm <= ", bflc::kMcMaxClients);
+    TORCH_CHECK(max_n_val > 0, "max_n_val must be positive");
+    TORCH_CHECK(x_maps.is_cuda() && x_maps.nbytes() >= bflc::kMcMaxClients * ctm && w_maps.is_cuda() &&
+                w_maps.nbytes() >= 2 * bflc::kMcMaxClients * ctm,
+                "x_maps: one tensor map per client slot, w_maps: [2][", bflc::kMcMaxClients, "] (device)");
     bflc::McValArgs r;
-    r.n_val = n_val; r.in_dim = in_dim; r.hidden = hidden; r.n_classes = n_classes;
+    r.max_n_val = max_n_val; r.in_dim = in_dim; r.hidden = hidden; r.n_classes = n_classes;
     r.max_cand = max_cand; r.max_comm = max_comm;
     r.plan = P<const bflc::McPlan>(plan_ptr);
     r.correct = P<unsigned int>(correct_ptr);
@@ -91,16 +117,11 @@ void bind_mc(py::module_& m) {
     r.w_maps = reinterpret_cast<const CUtensorMap*>(w_maps.data_ptr());
     r.clients = P<const bflc::McClients>(clients_ptr);
     r.b1_off = b1_off; r.b2_off = b2_off;
-    r.labels = labels.data_ptr<int32_t>(); r.labels_stride = labels_stride;
-    if (x_sf.has_value()) {
-      r.fp8 = true;
-      r.x_sf = x_sf->data_ptr<uint8_t>(); r.x_sf_stride = x_sf_stride;
-    }
+    r.fp8 = fp8;
     check(bflc::mc_val_sm100(r, cur_stream()), "mc_val_sm100");
   }, py::arg("plan_ptr"), py::arg("correct_ptr"), py::arg("x_maps"), py::arg("w_maps"), py::arg("clients_ptr"),
-     py::arg("b1_off"), py::arg("b2_off"), py::arg("labels"), py::arg("labels_stride"), py::arg("n_val"),
-     py::arg("in_dim"), py::arg("hidden"), py::arg("n_classes"), py::arg("max_cand"), py::arg("max_comm"),
-     py::arg("x_sf") = py::none(), py::arg("x_sf_stride") = 0);
+     py::arg("b1_off"), py::arg("b2_off"), py::arg("max_n_val"), py::arg("in_dim"), py::arg("hidden"),
+     py::arg("n_classes"), py::arg("max_cand"), py::arg("max_comm"), py::arg("fp8") = false);
   // TMA descriptor of a K-major operand [rows][K] (row pitch ld elements), box rows_tile x 128 B
   m.def("operand_map", [](int64_t ptr, int64_t ld, int rows, int K, bool fp8, int rows_tile) {
     CUtensorMap t;

@@ -4,6 +4,7 @@
 //
 //   k_mc_plan         QueryState for every client: trainer predicates, barrier words, Adam step
 //                     bases, committee list, simulated arrival order + first-K admission
+//                     (per-client shard sizes, step counts and validation rows: McClients)
 //   mlp_round x C     local training, one persistent launch per client (predicated)
 //   k_mc_byzantine    fault injection: update := global - s * (trained - global)
 //   mc_val            committee validation: every member x every admitted candidate, one launch
@@ -79,11 +80,21 @@ struct McBlockRecord {
   uint32_t pad;
 };
 
-// Per-client addresses, kept in device memory (one entry per client).
+// Per-client addresses and shard constants, kept in device memory (one entry per client),
+// written once at construction.  Clients may hold shards of different sizes: client c trains
+// steps[c] mini-batches of `batch` rows, reports n_samples[c] and validates as a committee member on
+// the first n_val[c] rows of its own shard.
 struct McClients {
   float* master[kMcMaxClients];            // fp32 work master (training weights, FedAvg operand)
   uint16_t* shadow[kMcMaxClients];         // bf16 work shadow
   uint8_t* blob[kMcMaxClients];            // fp8: Mx8MlpLayout blob (training copy + candidate)
+  const int32_t* labels[kMcMaxClients];    // the client's labels (validation reads [0, n_val))
+  const uint8_t* x_sf[kMcMaxClients];      // fp8: scale chunks of the client's inputs
+  uint32_t n_samples[kMcMaxClients];       // S_c = (rows_c / batch) * batch, the FedAvg weight
+  int steps[kMcMaxClients];                // training steps per round (loss terms = steps * batch)
+  int n_val[kMcMaxClients];                // validation rows of the client as a committee member
+  int batch;
+  int pad;
 };
 
 struct McArgs {
@@ -97,11 +108,12 @@ struct McArgs {
   long long n_params;
 };
 
-cudaError_t mc_plan_round(const McArgs& a, int steps_per_round, cudaStream_t s);
+// Adam step bases advance by each trainer's own McClients::steps
+cudaError_t mc_plan_round(const McArgs& a, cudaStream_t s);
 // byzantine clients (host list, ascending): if they trained, master/shadow := g - s * (w - g)
 cudaError_t mc_byzantine(const McArgs& a, const int* ids, int n_ids, float scale, cudaStream_t s);
-cudaError_t mc_consensus(const McArgs& a, int n_val, int n_samples, int n_loss_terms,
-                         int weight_by_score, cudaStream_t s);
+// scores, sample counts and average costs come from the per-client constants in McClients
+cudaError_t mc_consensus(const McArgs& a, int weight_by_score, cudaStream_t s);
 cudaError_t mc_fedavg(const McArgs& a, int n_clients, cudaStream_t s);
 // copy one blob to every client's blob slot (fp8: the quantised new global model)
 cudaError_t mc_broadcast_blob(const McArgs& a, const uint8_t* src, long long bytes, int n_clients,
@@ -109,20 +121,20 @@ cudaError_t mc_broadcast_blob(const McArgs& a, const uint8_t* src, long long byt
 
 // Committee validation of the multi-client round (mlp_val_sm100.cu, same chain body as
 // mlp_val_sm100): CTA (m-tile, candidate slot z, committee slot k) scores candidate plan->cand[z]
-// on the first n_val rows of member plan->comm[k] and adds the hits to
-// plan->correct[member][candidate].
+// on the first clients->n_val[member] rows of member plan->comm[k] (its own labels and, in fp8,
+// scale chunks) and adds the hits to plan->correct[member][candidate].  The grid spans the largest
+// client's tiles; a CTA past its member's n_val exits.
 struct McValArgs {
-  int n_val = 0, in_dim = 0, hidden = 0, n_classes = 0;
+  int max_n_val = 0;                       // max over clients of n_val: grid x = its 128-row tiles
+  int in_dim = 0, hidden = 0, n_classes = 0;
   int max_cand = 0, max_comm = 0;          // grid extent (slots beyond the plan's counts exit)
   const McPlan* plan = nullptr;
   unsigned int* correct = nullptr;         // &plan->correct[0][0]
-  const CUtensorMap* x_maps = nullptr;     // [client]: rows [0, n_val) of the client's inputs
+  const CUtensorMap* x_maps = nullptr;     // [client]: rows [0, n_val[client]) of the client's inputs
   const CUtensorMap* w_maps = nullptr;     // [layer][client] (bf16 shadows or fp8 blobs)
-  const McClients* clients = nullptr;      // bf16: biases from master; fp8: the blob
+  const McClients* clients = nullptr;      // candidate weights; the member's n_val, labels, x_sf
   long long b1_off = 0, b2_off = 0;        // bf16: element offsets of b1 / b2 in the master
-  const int32_t* labels = nullptr; long long labels_stride = 0;   // [client][rows]
   bool fp8 = false;
-  const uint8_t* x_sf = nullptr; long long x_sf_stride = 0;       // fp8: [client] scale chunks
 };
 cudaError_t mc_val_sm100(const McValArgs& r, cudaStream_t stream);
 

@@ -32,7 +32,7 @@ __device__ __forceinline__ uint32_t arrival_key(uint32_t seed, uint32_t epoch, u
 // chain order (C:239-244), i.e. whoever finishes first.  Clients sharing one GPU train one after
 // another, so there is no physical race to finish: the order is simulated as a permutation of the
 // trainers keyed by (seed, epoch, client), with every straggler after every other trainer.
-__global__ void k_mc_plan(McArgs a, int steps) {
+__global__ void k_mc_plan(McArgs a) {
   ptx::pdl_launch_dependents();
   ptx::pdl_wait();
   McState* st = a.st;
@@ -44,7 +44,7 @@ __global__ void k_mc_plan(McArgs a, int steps) {
     p->is_trainer[c] = tr ? 1 : 0;
     p->barrier[c] = 0u;
     p->opt_step[c] = p->opt_total[c];
-    if (tr) p->opt_total[c] += steps;
+    if (tr) p->opt_total[c] += a.clients->steps[c];
     p->loss_sum[c] = 0.f;
     p->train_correct[c] = 0u;
     for (int t = 0; t < kMcMaxClients; ++t) p->correct[c][t] = 0u;
@@ -102,9 +102,10 @@ struct McShared {
   ConsensusOut<kMcMaxClients> out;
 };
 
-// One block: scores = correct / n_val, run_consensus<32>, block record, ledger page.
+// One block: scores = correct / n_val of the scoring member, run_consensus<32> weighted by every
+// trainer's own sample count, block record, ledger page.
 __global__ void __launch_bounds__(kMcThreads)
-k_mc_consensus(McArgs a, int n_val, int n_samples, int n_loss_terms, int weight_by_score) {
+k_mc_consensus(McArgs a, int weight_by_score) {
   __shared__ McShared sh;
   ptx::pdl_launch_dependents();
   ptx::pdl_wait();
@@ -115,12 +116,12 @@ k_mc_consensus(McArgs a, int n_val, int n_samples, int n_loss_terms, int weight_
   const uint32_t adm = p->admitted_mask;
   ConsensusIn<kMcMaxClients>& in = sh.in;
   McBlockRecord* rec = a.ring + (epoch % static_cast<uint32_t>(a.ring_slots));
-  const float inv_n = 1.f / static_cast<float>(n_val > 0 ? n_val : 1);
+  const McClients* cl = a.clients;
   for (int i = threadIdx.x; i < kMcMaxClients * kMcMaxClients; i += blockDim.x) {
     const int r = i / kMcMaxClients, t = i % kMcMaxClients;
     const bool ok = r < n && t < n && (st->role[r] & ROLE_COMM) && (st->role[t] & ROLE_TRAINER) && ((adm >> t) & 1u);
     in.scored[r][t] = ok ? 1 : 0;
-    in.score[r][t] = ok ? static_cast<float>(p->correct[r][t]) * inv_n : 0.f;
+    in.score[r][t] = ok ? static_cast<float>(p->correct[r][t]) * (1.f / static_cast<float>(cl->n_val[r])) : 0.f;
     rec->score_rows[r][t] = in.score[r][t];
   }
   if (threadIdx.x < kMcMaxClients) {
@@ -128,8 +129,8 @@ k_mc_consensus(McArgs a, int n_val, int n_samples, int n_loss_terms, int weight_
     const bool tr = r < n && (st->role[r] & ROLE_TRAINER);
     in.role[r] = r < n ? st->role[r] : 0u;
     in.admitted[r] = (tr && ((adm >> r) & 1u)) ? 1 : 0;
-    in.n_samples[r] = tr ? static_cast<uint32_t>(n_samples) : 0u;
-    in.avg_cost[r] = tr ? p->loss_sum[r] / static_cast<float>(n_loss_terms > 0 ? n_loss_terms : 1) : 0.f;
+    in.n_samples[r] = tr ? cl->n_samples[r] : 0u;
+    in.avg_cost[r] = tr ? p->loss_sum[r] / static_cast<float>(cl->steps[r] * cl->batch) : 0.f;
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -290,9 +291,9 @@ int mc_grid(long long n_vec, int cap) {
 
 }  // namespace
 
-cudaError_t mc_plan_round(const McArgs& a, int steps_per_round, cudaStream_t s) {
+cudaError_t mc_plan_round(const McArgs& a, cudaStream_t s) {
   note_launch();
-  return launch_pdl(k_mc_plan, dim3(1), dim3(32), 0, s, a, steps_per_round);
+  return launch_pdl(k_mc_plan, dim3(1), dim3(32), 0, s, a);
 }
 
 cudaError_t mc_byzantine(const McArgs& a, const int* ids, int n_ids, float scale, cudaStream_t s) {
@@ -304,11 +305,9 @@ cudaError_t mc_byzantine(const McArgs& a, const int* ids, int n_ids, float scale
   return launch_pdl(k_mc_byzantine, dim3(mc_grid(a.n_params / 4, 64), n_ids), dim3(kMcThreads), 0, s, a, b, scale);
 }
 
-cudaError_t mc_consensus(const McArgs& a, int n_val, int n_samples, int n_loss_terms, int weight_by_score,
-                         cudaStream_t s) {
+cudaError_t mc_consensus(const McArgs& a, int weight_by_score, cudaStream_t s) {
   note_launch();
-  return launch_pdl(k_mc_consensus, dim3(1), dim3(kMcThreads), 0, s, a, n_val, n_samples, n_loss_terms,
-                    weight_by_score);
+  return launch_pdl(k_mc_consensus, dim3(1), dim3(kMcThreads), 0, s, a, weight_by_score);
 }
 
 cudaError_t mc_fedavg(const McArgs& a, int n_clients, cudaStream_t s) {

@@ -404,14 +404,13 @@ mlp_val_kernel(const __grid_constant__ CUtensorMap tmX, const ValArgs v) {
 // Multi-client committee validation (engine/multiclient.py): CTA (m-tile, candidate slot z,
 // committee slot k).  Who is candidate z and member k comes from the round plan; the candidate is
 // read in place from its client's buffers (bf16 work shadow + fp32 biases, or the fp8 blob), the
-// rows are the first n_val rows of the member's own shard.
+// rows are the first n_val[member] rows of the member's own shard.  Members may hold different
+// row counts: the grid spans the largest one, tiles past a member's n_val exit.
 struct McVal {
-  int n_val, in_dim, n_classes;
+  int in_dim, n_classes;
   const McPlan* plan; unsigned int* correct;
   const CUtensorMap* x_maps; const CUtensorMap* w_maps;
   const McClients* clients; long long b1_off, b2_off;
-  const int32_t* labels; long long labels_stride;
-  const uint8_t* x_sf; long long x_sf_stride;
   Mx8MlpLayout ql;
 };
 
@@ -425,11 +424,13 @@ mc_val_kernel(const McVal v) {
   const int z = blockIdx.y, k = blockIdx.z, m0 = blockIdx.x * kBM;
   const uint32_t tmem_base = val_setup(S, nullptr);
   ptx::pdl_wait();
-  if (z >= v.plan->n_cand || k >= v.plan->n_comm) {
+  const int member = k < v.plan->n_comm ? v.plan->comm[k] : 0;
+  const int n_val = v.clients->n_val[member];
+  if (z >= v.plan->n_cand || k >= v.plan->n_comm || m0 >= n_val) {
     if (warp == 1) ptx::tmem_dealloc(tmem_base, kTmemCols);
     return;
   }
-  const int member = v.plan->comm[k], cand = v.plan->cand[z];
+  const int cand = v.plan->cand[z];
   ChainJob j;
   j.tx = v.x_maps + member;
   j.m1 = v.w_maps + cand;
@@ -437,11 +438,11 @@ mc_val_kernel(const McVal v) {
   j.b1 = FP8 ? nullptr : v.clients->master[cand] + v.b1_off;
   j.b2 = FP8 ? nullptr : v.clients->master[cand] + v.b2_off;
   j.blob = FP8 ? v.clients->blob[cand] : nullptr;
-  j.x_sf = FP8 ? v.x_sf + member * v.x_sf_stride : nullptr;
-  j.labels = v.labels + member * v.labels_stride;
+  j.x_sf = FP8 ? v.clients->x_sf[member] : nullptr;
+  j.labels = v.clients->labels[member];
   j.correct = v.correct + member * kMcMaxClients + cand;
   j.wait_flag = nullptr; j.wait_value = 0u;
-  val_chain<FP8>(S, tmem_base, j, m0, v.n_val, v.in_dim, v.n_classes, v.ql);
+  val_chain<FP8>(S, tmem_base, j, m0, n_val, v.in_dim, v.n_classes, v.ql);
   val_teardown(tmem_base);
 }
 
@@ -485,18 +486,15 @@ cudaError_t mlp_val_sm100(const MlpValArgs& r, cudaStream_t stream) {
 
 cudaError_t mc_val_sm100(const McValArgs& r, cudaStream_t stream) {
   bind_context_once();
-  if (r.hidden != kChainH || r.n_classes > 64 || r.in_dim % 8 || r.n_val <= 0 || r.max_cand <= 0 ||
+  if (r.hidden != kChainH || r.n_classes > 64 || r.in_dim % 8 || r.max_n_val <= 0 || r.max_cand <= 0 ||
       r.max_cand > kMcMaxClients || r.max_comm <= 0 || r.max_comm > kMcMaxClients || r.plan == nullptr ||
-      r.correct == nullptr || r.x_maps == nullptr || r.w_maps == nullptr || r.clients == nullptr ||
-      r.labels == nullptr)
+      r.correct == nullptr || r.x_maps == nullptr || r.w_maps == nullptr || r.clients == nullptr)
     return cudaErrorInvalidValue;
-  if (r.fp8 && (r.x_sf == nullptr || r.in_dim % 16)) return cudaErrorInvalidValue;
+  if (r.fp8 && r.in_dim % 16) return cudaErrorInvalidValue;
   McVal v{};
-  v.n_val = r.n_val; v.in_dim = r.in_dim; v.n_classes = r.n_classes;
+  v.in_dim = r.in_dim; v.n_classes = r.n_classes;
   v.plan = r.plan; v.correct = r.correct; v.x_maps = r.x_maps; v.w_maps = r.w_maps;
   v.clients = r.clients; v.b1_off = r.b1_off; v.b2_off = r.b2_off;
-  v.labels = r.labels; v.labels_stride = r.labels_stride;
-  v.x_sf = r.x_sf; v.x_sf_stride = r.x_sf_stride;
   v.ql = mx8_mlp_layout(r.in_dim, r.hidden);
   static bool configured[2] = {false, false};
   cudaError_t e;
@@ -507,7 +505,7 @@ cudaError_t mc_val_sm100(const McValArgs& r, cudaStream_t stream) {
     configured[r.fp8 ? 1 : 0] = true;
   }
   note_launch();
-  const dim3 grid((r.n_val + kBM - 1) / kBM, r.max_cand, r.max_comm);
+  const dim3 grid((r.max_n_val + kBM - 1) / kBM, r.max_cand, r.max_comm);
   if (r.fp8) return launch_pdl(mc_val_kernel<true>, grid, dim3(kThreads), kValSmem, stream, v);
   return launch_pdl(mc_val_kernel<false>, grid, dim3(kThreads), kValSmem, stream, v);
 }

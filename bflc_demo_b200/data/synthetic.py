@@ -10,7 +10,7 @@ models genuinely learn and committee scores separate honest from Byzantine updat
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -33,21 +33,56 @@ def _label_split(n: int, n_classes: int, clients: int, alpha: float, rng: np.ran
     return [rng.dirichlet(np.full(n_classes, alpha)) for _ in range(clients)]
 
 
-def femnist_like(clients: int, samples_per_client: int, *, seed: int = 0, alpha: float = 0.0,
-                 n_classes: int = 62, hw: int = 28, noise: float = 48.0,
-                 only: Optional[int] = None) -> List[Shard]:
+def client_sizes(clients: int, mean: int, *, sigma: float, multiple: int = 1, seed: int = 0) -> List[int]:
+    """Seeded log-normal shard sizes (unequal clients, as FEMNIST writers are): client i holds a
+    multiple of ``multiple`` rows, at least one multiple, and the sizes add up to ``clients`` times
+    ``mean`` rounded to a multiple, so a skewed run trains as many samples as an equal one.
+    ``sigma = 0`` gives equal sizes."""
+    if clients <= 0 or multiple <= 0 or sigma < 0:
+        raise ValueError("client_sizes: clients > 0, multiple > 0, sigma >= 0")
+    unit = max(int(round(mean / multiple)), 1)                 # per-client mean, in multiples
+    total = clients * unit
+    z = np.random.default_rng([seed, 7919]).normal(0.0, 1.0, size=clients)
+    share = np.exp(sigma * z)
+    ideal = share / share.sum() * total
+    units = np.maximum(np.floor(ideal), 1).astype(np.int64)
+    # largest remainders first up to the total; over it (the one-multiple floor): trim the largest
+    frac_order = np.argsort(-(ideal - np.floor(ideal)), kind="stable")
+    i = 0
+    while units.sum() < total:
+        units[frac_order[i % clients]] += 1
+        i += 1
+    while units.sum() > total and units.max() > 1:
+        units[int(np.argmax(units))] -= 1
+    return [int(u) * multiple for u in units]
+
+
+def femnist_like(clients: Optional[int] = None, samples_per_client: Optional[int] = None, *, seed: int = 0,
+                 alpha: float = 0.0, n_classes: int = 62, hw: int = 28, noise: float = 48.0,
+                 only: Optional[int] = None, sizes: Optional[Sequence[int]] = None) -> List[Shard]:
     """uint8 [n, hw*hw] images: class prototype (0..255) + Gaussian pixel noise.  The class
     prototypes depend only on ``seed``; client ``i``'s samples only on ``(seed, i)``, so a
-    rank can generate just its own shard with ``only=i`` (returns a 1-element list)."""
+    rank can generate just its own shard with ``only=i`` (returns a 1-element list).
+    ``sizes``: client ``i`` draws ``sizes[i]`` samples instead of ``samples_per_client``
+    (``clients`` defaults to ``len(sizes)``); ``alpha > 0`` skews every client's label mix."""
+    if sizes is not None:
+        sizes = [int(v) for v in sizes]
+        if clients is None:
+            clients = len(sizes)
+        if len(sizes) != clients or any(v <= 0 for v in sizes):
+            raise ValueError(f"femnist_like: need {clients} positive sizes, got {sizes}")
+    elif clients is None or samples_per_client is None:
+        raise ValueError("femnist_like: give clients and samples_per_client, or sizes")
     protos = np.random.default_rng(seed).integers(0, 256, size=(n_classes, hw * hw)).astype(np.float32)
     out = []
     for i in range(clients):
         if only is not None and i != only:
             continue
+        n_i = sizes[i] if sizes is not None else samples_per_client
         rng = np.random.default_rng([seed, 1000 + i])
-        p = _label_split(samples_per_client, n_classes, 1, alpha, rng)[0]
-        y = rng.choice(n_classes, size=samples_per_client, p=p)
-        x = protos[y] + rng.normal(0, noise, size=(samples_per_client, hw * hw)).astype(np.float32)
+        p = _label_split(n_i, n_classes, 1, alpha, rng)[0]
+        y = rng.choice(n_classes, size=n_i, p=p)
+        x = protos[y] + rng.normal(0, noise, size=(n_i, hw * hw)).astype(np.float32)
         x = np.clip(x, 0, 255).astype(np.uint8)
         out.append(Shard(torch.from_numpy(x), torch.from_numpy(y.astype(np.int64)), n_classes))
     return out

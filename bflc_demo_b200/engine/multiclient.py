@@ -14,12 +14,18 @@ matches ``FusedEngine`` so callers can swap engines.
     k_mc_byzantine         fault injection: update := global - s * (trained - global)
     [fp8] quantize x C     each client's candidate blob from its trained master
     mc_val                 every committee member scores every admitted candidate on its own
-                           n_val rows: ONE launch over (m-tile, candidate, member)
+                           n_val_c rows: ONE launch over (m-tile, candidate, member)
     k_mc_consensus         scores, run_consensus<32>, ledger page, block record
     k_mc_fedavg            deterministic FedAvg into the global model and every client
     [fp8] quantize + k_mc_bcast   the new global blob into every client's training copy
 
 Every trainer trains, also those that will not be admitted (the reference rejects at upload).
+
+Clients may hold shards of different sizes (and label mixes).  Client c with rows_c rows trains
+S_c = (rows_c // B) * B samples in steps_c = S_c / B * local_epochs steps, validates as a committee
+member on n_val_c = min(val_samples or rows_c, rows_c) rows of its own shard and reports
+n_samples = S_c, so FedAvg weights the selected clients by their sample counts -- the rule
+``FusedEngine`` applies per rank.  These constants live in the device-resident ``McClients``.
 """
 from __future__ import annotations
 
@@ -63,26 +69,43 @@ class MultiClientEngine:
         assert sz["McState"] == _MC_STATE.size and sz["McBlockRecord"] == _MC_REC.size, \
             "multi-client struct layout changed: update _MC_STATE / _MC_REC"
 
-        rows, n_classes = len(shards[0]), shards[0].n_classes
-        if any(len(s) != rows or s.n_classes != n_classes for s in shards):
-            raise ValueError("every client shard must have the same size and class count")
-        self.in_dim = shards[0].x.reshape(rows, -1).shape[1]
+        n_classes = shards[0].n_classes
+        B = cfg.batch_size
+        self.fp8 = cfg.dtype == "fp8"
+        rows_c = [len(s) for s in shards]
+        for c, s in enumerate(shards):
+            if s.n_classes != n_classes:
+                raise ValueError(f"client {c} has {s.n_classes} classes, client 0 has {n_classes}: "
+                                 "every shard must have the same class count")
+            if rows_c[c] < B:
+                raise ValueError(f"client {c} holds {rows_c[c]} rows, fewer than one batch ({B})")
+            if self.fp8 and rows_c[c] % 128:
+                raise ValueError(f"dtype='fp8' needs shard rows % 128 == 0; client {c} holds {rows_c[c]}")
+        self.in_dim = shards[0].x.reshape(rows_c[0], -1).shape[1]
+        if any(s.x.reshape(len(s), -1).shape[1] != self.in_dim for s in shards):
+            raise ValueError("every client shard must have the same feature size")
         self.spec = mlp_spec(self.in_dim, cfg.hidden, n_classes)
         self.n_params = P = self.spec.total
         self.n_classes = n_classes
-        B = cfg.batch_size
-        self.S = (rows // B) * B
-        self.steps = (self.S // B) * cfg.local_epochs
-        self.rows = rows
-        self.n_val = min(cfg.val_samples or rows, rows)
-        self.fp8 = cfg.dtype == "fp8"
+        # per-client shard constants (the same rule as FusedEngine applies per rank)
+        self.rows_per_client = rows_c
+        self.samples_per_client = [(r // B) * B for r in rows_c]
+        self.steps_per_client = [(S // B) * cfg.local_epochs for S in self.samples_per_client]
+        self.n_val_per_client = [min(cfg.val_samples or r, r) for r in rows_c]
+        # equal shards: the scalars of a uniform engine; unequal shards: None (use the lists)
+        def uniform(v):
+            return v[0] if all(x == v[0] for x in v) else None
+        self.rows = uniform(self.rows_per_client)
+        self.S = uniform(self.samples_per_client)
+        self.steps = uniform(self.steps_per_client)
+        self.n_val = uniform(self.n_val_per_client)
         if cfg.dtype not in ("bf16", "fp8"):
             raise ValueError("MultiClientEngine: dtype must be bf16 or fp8")
         if not (cfg.hidden == 256 and n_classes <= 64 and self.in_dim % 16 == 0):
             raise ValueError("MultiClientEngine runs the flagship MLP: hidden == 256, <= 64 classes, "
                              "in_dim % 16 == 0")
-        if self.fp8 and not (B % 128 == 0 and rows % 128 == 0):
-            raise ValueError("dtype='fp8' needs batch % 128 == 0 and shard rows % 128 == 0")
+        if self.fp8 and B % 128:
+            raise ValueError("dtype='fp8' needs batch % 128 == 0")
 
         # ---- per-client model state: [C, P] master / shadow / grad, own Adam moments ---------
         dev = self.dev
@@ -129,34 +152,48 @@ class MultiClientEngine:
                          optimizer=cfg.optimizer, lr=cfg.learning_rate,
                          loss_sum=self.loss_sum[c:c + 1], correct=self.train_correct[c:c + 1],
                          step_dev_ptr=pp + sz["mc_plan_opt_step_off"] + 4 * c, fp8=self.fp8)
-            if not tr.fused_ok(self.steps):
+            if not tr.fused_ok(self.steps_per_client[c]):
                 raise ValueError("shape outside the persistent trainer's limits")
             self.trainers.append(tr)
         self.ql = m.mx8_mlp_layout(self.in_dim, cfg.hidden) if self.fp8 else None
-        blobs = [t.work_q.data_ptr() for t in self.trainers] if self.fp8 else []
-        self.clients_dev = torch.frombuffer(bytearray(m.mc_clients_bytes(
-            [self.master[c].data_ptr() for c in range(n)], [self.shadow[c].data_ptr() for c in range(n)],
-            blobs)), dtype=torch.uint8).to(dev)
-        self.args = dict(st=self.state_bytes.data_ptr(), plan=pp, ring=self.ring_bytes.data_ptr(),
-                         ring_slots=cfg.ring_slots, clients=self.clients_dev.data_ptr(),
-                         global_master=self.global_master.data_ptr(),
-                         global_shadow=self.global_shadow.data_ptr(), n_params=P)
         self.byz_ids = sorted(r for r in set(cfg.byzantine_ranks) if 0 <= r < n)
 
-        # ---- resident inputs, converted once ---------------------------------------------------
+        # ---- resident inputs, converted once: one ragged allocation per tensor, client c's rows
+        #      at a 128-row aligned offset, exposed as per-client views x_bf[c], y[c], x_q[c], x_sf[c]
         D = self.in_dim
-        self.x_bf = torch.empty(n, rows, D, device=dev, dtype=torch.bfloat16)
-        self.y = torch.empty(n, rows, device=dev, dtype=torch.int32)
-        self.sf_stride = sf_bytes(rows, D)
-        self.x_q = torch.zeros(n, rows, D, device=dev, dtype=torch.uint8) if self.fp8 else None
-        self.x_sf = torch.full((n, self.sf_stride), 127, device=dev, dtype=torch.uint8) if self.fp8 else None
+        row_off, sf_off, r0, f0 = [], [], 0, 0
+        for r in rows_c:
+            row_off.append(r0)
+            sf_off.append(f0)
+            r0 += -(-r // 128) * 128
+            f0 += sf_bytes(r, D)
+        x_bf_all = torch.empty(r0, D, device=dev, dtype=torch.bfloat16)
+        y_all = torch.zeros(r0, device=dev, dtype=torch.int32)
+        x_q_all = torch.zeros(r0, D, device=dev, dtype=torch.uint8) if self.fp8 else None
+        x_sf_all = torch.full((f0,), 127, device=dev, dtype=torch.uint8) if self.fp8 else None
+        self.x_bf = [x_bf_all[o:o + r] for o, r in zip(row_off, rows_c)]
+        self.y = [y_all[o:o + r] for o, r in zip(row_off, rows_c)]
+        self.x_q = [x_q_all[o:o + r] for o, r in zip(row_off, rows_c)] if self.fp8 else None
+        self.x_sf = [x_sf_all[o:o + sf_bytes(r, D)] for o, r in zip(sf_off, rows_c)] if self.fp8 else None
         for c, s in enumerate(shards):
-            xu = s.x.reshape(rows, -1).to(dev, torch.uint8).contiguous()
+            xu = s.x.reshape(rows_c[c], -1).to(dev, torch.uint8).contiguous()
             m.prep_inputs(xu, self.x_bf[c], self.x_q[c] if self.fp8 else None,
                           self.x_sf[c] if self.fp8 else None, 1.0 / 255.0)
             self.y[c].copy_(s.y.to(torch.int32))
 
-        # ---- validation tensor maps: x of every client (its first n_val rows), [layer][client]
+        blobs = [t.work_q.data_ptr() for t in self.trainers] if self.fp8 else []
+        self.clients_dev = torch.frombuffer(bytearray(m.mc_clients_bytes(
+            [self.master[c].data_ptr() for c in range(n)], [self.shadow[c].data_ptr() for c in range(n)],
+            blobs, [self.y[c].data_ptr() for c in range(n)],
+            [self.x_sf[c].data_ptr() for c in range(n)] if self.fp8 else [],
+            self.samples_per_client, self.steps_per_client, self.n_val_per_client, B)),
+            dtype=torch.uint8).to(dev)
+        self.args = dict(st=self.state_bytes.data_ptr(), plan=pp, ring=self.ring_bytes.data_ptr(),
+                         ring_slots=cfg.ring_slots, clients=self.clients_dev.data_ptr(),
+                         global_master=self.global_master.data_ptr(),
+                         global_shadow=self.global_shadow.data_ptr(), n_params=P)
+
+        # ---- validation tensor maps: x of every client (its first n_val_c rows), [layer][client]
         #      weights read in place (bf16 work shadow, or the client's fp8 blob) --------------
         K = MAX_CLIENTS
         CTM = sz["CUtensorMap"]
@@ -164,7 +201,8 @@ class MultiClientEngine:
         e1, e2 = self.spec.by_name["w1"], self.spec.by_name["w2"]
         for c in range(n):
             xsrc = self.x_q[c] if self.fp8 else self.x_bf[c]
-            xm[c * CTM:(c + 1) * CTM] = m.operand_map(xsrc.data_ptr(), D, self.n_val, D, self.fp8, 128)
+            xm[c * CTM:(c + 1) * CTM] = m.operand_map(xsrc.data_ptr(), D, self.n_val_per_client[c], D,
+                                                      self.fp8, 128)
             if self.fp8:
                 base = self.trainers[c].work_q.data_ptr()
                 w1 = m.gemm_b_map(base + self.ql["w1q"], e1.shape[0], D, D, False, True, G.EPI_GENERIC, 256)
@@ -199,10 +237,10 @@ class MultiClientEngine:
     def phase_train(self):
         """Plan + local training of every trainer (+ Byzantine injection, + candidate blobs)."""
         m, cfg, sz = self.mod, self.cfg, self.sz
-        m.mc_plan_round(self.args, self.steps)
+        m.mc_plan_round(self.args)
         for c, tr in enumerate(self.trainers):
             m.set_predicate(self.plan_ptr + sz["mc_plan_is_trainer_off"] + 4 * c)
-            tr.train_epoch_fused(self.x_bf[c], self.y[c], self.steps,
+            tr.train_epoch_fused(self.x_bf[c], self.y[c], self.steps_per_client[c],
                                  self.plan_ptr + sz["mc_plan_barrier_off"] + 4 * c,
                                  x_q=self.x_q[c] if self.fp8 else None,
                                  x_sf=self.x_sf[c] if self.fp8 else None)
@@ -219,14 +257,13 @@ class MultiClientEngine:
         m, sz = self.mod, self.sz
         e = self.spec.by_name
         m.mc_val(self.plan_ptr, self.plan_ptr + sz["mc_plan_correct_off"], self.x_maps, self.w_maps,
-                 self.clients_dev.data_ptr(), e["b1"].offset, e["b2"].offset, self.y, self.rows,
-                 self.n_val, self.in_dim, self.cfg.hidden, self.n_classes, self.max_cand,
-                 self.cfg.committee_size, self.x_sf if self.fp8 else None, self.sf_stride)
+                 self.clients_dev.data_ptr(), e["b1"].offset, e["b2"].offset, max(self.n_val_per_client),
+                 self.in_dim, self.cfg.hidden, self.n_classes, self.max_cand, self.cfg.committee_size, self.fp8)
 
     def phase_aggregate(self):
         """Consensus, ledger page, block record, FedAvg into the global model and every client."""
         m, cfg = self.mod, self.cfg
-        m.mc_consensus(self.args, self.n_val, self.S, self.steps * cfg.batch_size, cfg.weight_by_score)
+        m.mc_consensus(self.args, cfg.weight_by_score)
         m.mc_fedavg(self.args, cfg.clients)
         if self.fp8:
             self._broadcast_global_blob()
@@ -273,13 +310,16 @@ class MultiClientEngine:
                     selected_mask=f[73], global_loss=f[74], model_digest=f[76])
 
     def drain_blocks(self) -> List[str]:
-        """Finished McBlockRecords -> host C++ ledger, which re-executes every election.
+        """Finished McBlockRecords -> host C++ ledger, which re-executes every election.  The
+        device's FedAvg weight of every selected client must equal the host block's bit for bit
+        (both sides compute it in double in the shared run_consensus).
         Returns the mismatches ([] = device and host agree)."""
         torch.cuda.synchronize()
         st = self.read_state()
         ring = bytes(self.ring_bytes.cpu().numpy())
         rs, n, K = _MC_REC.size, self.cfg.clients, MAX_CLIENTS
         errs: List[str] = []
+        dev_weights: List[tuple] = []          # (epoch, record weight[0..n)) of appended blocks
         while self.drained < st["epoch"]:
             e = self.drained
             f = _MC_REC.unpack_from(ring, (e % self.cfg.ring_slots) * rs)
@@ -291,7 +331,7 @@ class MultiClientEngine:
             p += K                                   # median
             n_samples = f[p:p + n]; p += K
             avg_cost = f[p:p + n]; p += K
-            p += K                                   # weight
+            weight = f[p:p + n]; p += K
             adm, sel, gl, wbs, digest, seq = f[p:p + 6]
             if f[0] != e or seq != e + 1:
                 errs.append(f"ring slot for epoch {e} holds epoch {f[0]} seq {seq}")
@@ -304,7 +344,18 @@ class MultiClientEngine:
             if msg:
                 errs.append(f"epoch {e}: {msg}")
                 break
+            dev_weights.append((e, weight))
             self.drained += 1
+        if dev_weights:
+            blocks = self.host_ledger.blocks()[-len(dev_weights):]
+            for (e, weight), blk in zip(dev_weights, blocks):
+                if blk["epoch"] != e:
+                    errs.append(f"epoch {e}: host block holds epoch {blk['epoch']}")
+                    continue
+                for t, w in zip(blk["selected"], blk["weight"]):
+                    if weight[t] != w:
+                        errs.append(f"epoch {e}: FedAvg weight of client {t}: device {weight[t]!r} "
+                                    f"host {w!r}")
         return errs
 
     def committee(self) -> List[int]:

@@ -3,6 +3,7 @@ reference, python-sdk/main.py:343-358, for one NVSwitch box):
 
     python -m bflc_demo_b200.run --model mlp --rounds 20                       # 1 GPU, solo
     python -m bflc_demo_b200.run --clients 20 --rounds 20     # 20 clients on 1 GPU (20/4/10/6)
+    python -m bflc_demo_b200.run --clients 20 --alpha 0.5 --size-sigma 0.8    # skewed labels + sizes
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 \\
         -m bflc_demo_b200.run --model resnet18 --rounds 5 --byzantine 7       # config #4
 
@@ -22,7 +23,7 @@ import torch
 import torch.distributed as dist
 
 from .config import FLConfig
-from .data.synthetic import cifar_like, femnist_like, tokens_like
+from .data.synthetic import cifar_like, client_sizes, femnist_like, tokens_like
 from .utils.metrics import RunLog
 from .utils.tracing import PhaseTimer
 
@@ -49,6 +50,11 @@ def main(argv=None):
     ap.add_argument("--committee", type=int, default=4, help="--clients: committee size (COMM_COUNT)")
     ap.add_argument("--needed", type=int, default=10, help="--clients: NEEDED_UPDATE_COUNT")
     ap.add_argument("--aggregate", type=int, default=6, help="--clients: AGGREGATE_COUNT")
+    ap.add_argument("--alpha", type=float, default=0.0,
+                    help="--clients: Dirichlet label skew of every client (0 = IID)")
+    ap.add_argument("--size-sigma", type=float, default=0.0,
+                    help="--clients: log-normal spread of the shard sizes (0 = equal shards; the "
+                         "total stays clients x samples)")
     a = ap.parse_args(argv)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -127,10 +133,14 @@ def run_multiclient(a):
     cfg = FLConfig(clients=a.clients, committee_size=a.committee, needed_updates=a.needed,
                    aggregate_count=a.aggregate, batch_size=B, samples_per_client=S, learning_rate=LR,
                    optimizer=a.optimizer, byzantine_ranks=a.byzantine, ring_slots=1024,
-                   dtype=a.dtype).validate()
-    shards = femnist_like(a.clients, S, seed=7)
+                   dtype=a.dtype, non_iid_alpha=a.alpha).validate()
+    # shard sizes in whole batches (every client trains at least one; fp8 batches are 128-row tiles)
+    sizes = client_sizes(a.clients, S, sigma=a.size_sigma, multiple=B, seed=7) if a.size_sigma > 0 else None
+    shards = femnist_like(a.clients, S, seed=7, alpha=cfg.non_iid_alpha, sizes=sizes)
     test = femnist_like(1, 2048, seed=7, only=0)[0]
     eng = MultiClientEngine(cfg, shards, device=0)
+    print(f"[clients] alpha {cfg.non_iid_alpha} size_sigma {a.size_sigma} rows per client "
+          f"{eng.rows_per_client}")
     eng.capture()
     log = RunLog(rank=0)
     timer = PhaseTimer()
@@ -142,7 +152,8 @@ def run_multiclient(a):
         log.round(st["epoch"] - 1, st["global_loss"], test_acc=eng.evaluate(test),
                   committee=[r for r, x in enumerate(st["roles"]) if x & 2])
     errs = eng.drain_blocks()
-    summary = dict(rounds=a.rounds, clients=a.clients, wall_s=round(time.time() - t0, 3),
+    summary = dict(rounds=a.rounds, clients=a.clients, alpha=cfg.non_iid_alpha, size_sigma=a.size_sigma,
+                   rows_per_client=eng.rows_per_client, wall_s=round(time.time() - t0, 3),
                    timing=timer.summary(), ledger_mismatches=errs, chain_ok=eng.host_ledger.verify_chain(),
                    blocks=eng.host_ledger.n_blocks(), launches_per_round=eng.launches_per_round)
     print("SUMMARY " + json.dumps(summary))

@@ -1,12 +1,17 @@
 """Rounds/s of the multi-client engine (engine/multiclient.py) on one GPU.
 
-    python scripts/bench_multiclient.py [--clients 8 20 32] [--steps 20] [--warmup 5]
+    python scripts/bench_multiclient.py [--clients 8 20 32] [--skewed 20] [--size-sigma 0.8]
+                                        [--steps 20] [--warmup 5]
 
 For C clients (committee / needed / aggregate in the reference's 20 / 4 / 10 / 6 proportions),
 4096 samples and batch 512 per client, fp8 + Adam and bf16 + SGD: device-event time of the
 captured round graph with an L2 flush between timed rounds (as bench.py), the split into
 training / validation / consensus + FedAvg (the same round captured as three graphs), and FedAvg
 alone against the HBM roofline.  Prints one JSON line per configuration.
+
+``--skewed C``: the same C-client workload with unequal shards -- log-normal sizes
+(``client_sizes``, ``--size-sigma``) in whole batches with the same total sample count (C x 4096),
+so training time is comparable; the validation grid spans the largest member's rows.
 """
 from __future__ import annotations
 
@@ -21,7 +26,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from bflc_demo_b200.config import FLConfig  # noqa: E402
-from bflc_demo_b200.data.synthetic import femnist_like  # noqa: E402
+from bflc_demo_b200.data.synthetic import client_sizes, femnist_like  # noqa: E402
 from bflc_demo_b200.engine.multiclient import MultiClientEngine  # noqa: E402
 
 HBM_PEAK = 7.7e12   # HBM3e bandwidth of one HGX B200 GPU, bytes/s (NVIDIA data sheet)
@@ -51,11 +56,12 @@ def timed(fn, flush, reps, stream):
     return ts[len(ts) // 2]
 
 
-def bench(clients, dtype, opt, steps, warmup, flush):
+def bench(clients, dtype, opt, steps, warmup, flush, size_sigma=0.0):
     cfg = FLConfig.reference_scaled(clients, model="mlp", dataset="femnist", hidden=256, batch_size=512,
                                     samples_per_client=4096, dtype=dtype, optimizer=opt,
                                     learning_rate=0.002 if opt == "adam" else 0.05, ring_slots=1024)
-    eng = MultiClientEngine(cfg, femnist_like(clients, 4096, seed=7), device=0)
+    sizes = client_sizes(clients, 4096, sigma=size_sigma, multiple=512, seed=7) if size_sigma > 0 else None
+    eng = MultiClientEngine(cfg, femnist_like(clients, 4096, seed=7, sizes=sizes), device=0)
     eng.capture()
     for _ in range(warmup):
         eng.run_round()
@@ -93,8 +99,10 @@ def bench(clients, dtype, opt, steps, warmup, flush):
     fedavg_us = timed(lambda: g.replay(), flush, steps, s)
     P = eng.n_params
     fed_bytes = n_sel * P * 4 + P * 6 + clients * P * 6
+    rows = eng.rows_per_client
     return dict(clients=clients, committee=cfg.committee_size, needed=cfg.needed_updates,
                 aggregate=cfg.aggregate_count, dtype=dtype, optimizer=opt, samples=4096, batch=512,
+                size_sigma=size_sigma, samples_total=sum(rows), rows_min=min(rows), rows_max=max(rows),
                 round_us=round(round_us, 1), rounds_per_s=round(1e6 / round_us, 1),
                 train_us=round(split[0], 1), validate_us=round(split[1], 1),
                 consensus_fedavg_us=round(split[2], 1), fedavg_us=round(fedavg_us, 1),
@@ -107,13 +115,17 @@ def main():
     ap.add_argument("--clients", type=int, nargs="*", default=[8, 20, 32])
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--skewed", type=int, nargs="*", default=[20],
+                    help="client counts also run with unequal shards (--size-sigma)")
+    ap.add_argument("--size-sigma", type=float, default=0.8)
     a = ap.parse_args()
     print(json.dumps(dict(gpu=torch.cuda.get_device_name(0), power_limit=power_limit(),
                           hbm_peak_bytes_per_s=HBM_PEAK)), flush=True)
     flush = torch.empty(256 << 20, device="cuda", dtype=torch.uint8)   # > L2
-    for c in a.clients:
+    runs = [(c, 0.0) for c in a.clients] + [(c, a.size_sigma) for c in a.skewed]
+    for c, sigma in runs:
         for dtype, opt in (("fp8", "adam"), ("bf16", "sgd")):
-            print(json.dumps(bench(c, dtype, opt, a.steps, a.warmup, flush)), flush=True)
+            print(json.dumps(bench(c, dtype, opt, a.steps, a.warmup, flush, sigma)), flush=True)
             torch.cuda.empty_cache()
 
 
