@@ -10,9 +10,12 @@ from __future__ import annotations
 
 import dataclasses
 import json
+import math
 import os
 from dataclasses import dataclass, field
 from typing import List, Optional
+
+SERVER_OPTIMIZERS = ("none", "momentum", "adam", "yogi")
 
 
 @dataclass
@@ -38,6 +41,13 @@ class FLConfig:
     optimizer: str = "sgd"            # sgd (M:127) | adam (commented alternative, M:126)
     dtype: str = "bf16"               # fp32 | bf16 | fp8
     non_iid_alpha: float = 0.0        # 0 = IID contiguous split (M:43-48); >0 Dirichlet skew
+    # ---- drift under skewed data (MultiClientEngine only; the other engines refuse them) ----
+    prox_mu: float = 0.0              # FedProx: local loss + mu/2 ||w - w_global||^2
+    server_optimizer: str = "none"    # none (FedAvg) | momentum (FedAvgM) | adam (FedAdam) | yogi (FedYogi)
+    server_lr: float = 1.0            # server step on the pseudo-gradient (average - global)
+    server_beta1: float = 0.9
+    server_beta2: float = 0.99
+    server_tau: float = 1e-3          # adaptivity; the second moment starts at tau^2
     # ---- faults (SURVEY.md 5.3) ----
     byzantine_ranks: List[int] = field(default_factory=list)
     byzantine_scale: float = 5.0
@@ -80,7 +90,31 @@ class FLConfig:
         for r in c.byzantine_ranks:
             if not (0 <= r < c.clients):
                 raise ValueError(f"byzantine rank {r} out of range")
+        if not (math.isfinite(c.prox_mu) and c.prox_mu >= 0):
+            raise ValueError("prox_mu must be finite and >= 0")
+        if c.server_optimizer not in SERVER_OPTIMIZERS:
+            raise ValueError("server_optimizer must be one of " + ", ".join(SERVER_OPTIMIZERS))
+        if not (c.server_lr > 0 and math.isfinite(c.server_lr)):
+            raise ValueError("server_lr must be > 0")
+        for name in ("server_beta1", "server_beta2"):
+            if not (0 <= getattr(c, name) < 1):
+                raise ValueError(f"{name} must be in [0, 1)")
+        if not (c.server_tau > 0 and math.isfinite(c.server_tau)):
+            raise ValueError("server_tau must be > 0")
         return self
+
+    @property
+    def plain_fedavg(self) -> bool:
+        """No proximal term and no server optimizer: the update rule of every engine."""
+        return self.prox_mu == 0 and self.server_optimizer == "none"
+
+    def require_plain_fedavg(self, engine: str) -> None:
+        """FedProx and the server optimizers exist in MultiClientEngine only; the other engines
+        refuse them rather than train something else than what was asked for."""
+        if not self.plain_fedavg:
+            raise ValueError(f"{engine} supports neither prox_mu > 0 nor a server optimizer "
+                             f"(prox_mu={self.prox_mu}, server_optimizer={self.server_optimizer!r}); "
+                             "use MultiClientEngine (run.py --clients N)")
 
     @property
     def n_trainers(self) -> int:

@@ -258,7 +258,7 @@ void bind_extra(py::module_& m) {
                         int64_t round_seq_ptr, const OptT& x_q, const OptT& x_sf, const OptT& work_q,
                         const OptT& h_q, const OptT& h_sf, const std::optional<py::dict>& fed,
                         std::vector<int64_t> upq_off, int n_samples, int n_loss_terms, int byz_mode,
-                        double byz_scale, int straggle_us) {
+                        double byz_scale, int straggle_us, double prox_mu, const OptT& prox_anchor) {
     TORCH_CHECK(offs.size() == 4, "offs = element offsets of w1, b1, w2, b2 in the flat buffer");
     bflc::MlpRoundArgs r;
     r.batch = batch; r.steps = steps; r.in_dim = in_dim; r.hidden = hidden; r.n_classes = n_classes;
@@ -302,6 +302,13 @@ void bind_extra(py::module_& m) {
       r.n_samples = n_samples; r.n_loss_terms = n_loss_terms; r.byz_mode = byz_mode; r.byz_scale = (float)byz_scale;
       r.straggle_us = straggle_us;
     }
+    if (prox_anchor.has_value()) {
+      TORCH_CHECK(prox_anchor->scalar_type() == at::kFloat && prox_anchor->numel() == master.numel() &&
+                  prox_anchor->is_contiguous() && prox_anchor->device() == master.device(),
+                  "prox_anchor: contiguous fp32 with the master's layout, on the master's device");
+      r.prox_anchor = prox_anchor->data_ptr<float>();
+    }
+    r.prox_mu = (float)prox_mu;
     check(bflc::mlp_round_sm100(r, cur_stream()), "mlp_round_sm100");
   }, py::arg("x"), py::arg("labels"), py::arg("master"), py::arg("shadow"), py::arg("grad"), py::arg("offs"),
      py::arg("h"), py::arg("dlogits"), py::arg("dh"), py::arg("loss_sum"), py::arg("correct"),
@@ -312,7 +319,7 @@ void bind_extra(py::module_& m) {
      py::arg("work_q") = py::none(), py::arg("h_q") = py::none(), py::arg("h_sf") = py::none(),
      py::arg("fed") = py::none(), py::arg("upq_off") = std::vector<int64_t>{}, py::arg("n_samples") = 0,
      py::arg("n_loss_terms") = 0, py::arg("byz_mode") = 0, py::arg("byz_scale") = 0.0,
-     py::arg("straggle_us") = 0);
+     py::arg("straggle_us") = 0, py::arg("prox_mu") = 0.0, py::arg("prox_anchor") = py::none());
   // committee validation of every candidate in one launch (fwd1 -> relu -> fwd2 -> argmax)
   m.def("mlp_val", [](at::Tensor x, at::Tensor labels, at::Tensor correct, at::Tensor maps,
                       int64_t dyn1_ptr, int64_t dyn2_ptr, int n_val, int in_dim, int hidden,

@@ -4,6 +4,7 @@
 
 #include <cstdint>
 #include <cstring>
+#include <string>
 
 #include "bflc_kernels.h"
 #include "mc_round.h"
@@ -90,9 +91,21 @@ void bind_mc(py::module_& m) {
   m.def("mc_consensus", [](const py::dict& d, bool weight_by_score) {
     check(bflc::mc_consensus(make_mc(d), weight_by_score ? 1 : 0, cur_stream()), "mc_consensus");
   });
-  m.def("mc_fedavg", [](const py::dict& d, int n_clients) {
-    check(bflc::mc_fedavg(make_mc(d), n_clients, cur_stream()), "mc_fedavg");
-  });
+  // server optimizer: "none" (plain FedAvg) | "momentum" | "adam" | "yogi"; m / v: device
+  // addresses of the fp32 [n_params] server state (v: adam and yogi only)
+  m.def("mc_fedavg", [](const py::dict& d, int n_clients, const std::string& server_optimizer, double lr,
+                        double beta1, double beta2, double tau, int64_t m_ptr, int64_t v_ptr) {
+    bflc::McServerOpt so;
+    if (server_optimizer == "none") so.mode = bflc::MC_SERVER_NONE;
+    else if (server_optimizer == "momentum") so.mode = bflc::MC_SERVER_MOMENTUM;
+    else if (server_optimizer == "adam") so.mode = bflc::MC_SERVER_ADAM;
+    else if (server_optimizer == "yogi") so.mode = bflc::MC_SERVER_YOGI;
+    else TORCH_CHECK(false, "server_optimizer must be none, momentum, adam or yogi, got ", server_optimizer);
+    so.lr = (float)lr; so.beta1 = (float)beta1; so.beta2 = (float)beta2; so.tau = (float)tau;
+    so.m = P<float>(m_ptr); so.v = P<float>(v_ptr);
+    check(bflc::mc_fedavg(make_mc(d), n_clients, cur_stream(), so), "mc_fedavg");
+  }, py::arg("args"), py::arg("n_clients"), py::arg("server_optimizer") = "none", py::arg("lr") = 1.0,
+     py::arg("beta1") = 0.9, py::arg("beta2") = 0.99, py::arg("tau") = 1e-3, py::arg("m") = 0, py::arg("v") = 0);
   m.def("mc_broadcast_blob", [](const py::dict& d, at::Tensor src, int n_clients) {
     check(bflc::mc_broadcast_blob(make_mc(d), src.data_ptr<uint8_t>(), src.numel(), n_clients, cur_stream()),
           "mc_broadcast_blob");

@@ -184,6 +184,12 @@ struct MlpRoundArgs {
   int n_samples = 0, n_loss_terms = 0, byz_mode = 0;
   float byz_scale = 0.f;
   int straggle_us = 0;   // fault injection: publish this late (first-K-wins admission test)
+  // ---- FedProx: every optimizer update uses g' = fmaf(prox_mu, w - anchor, g), w = the master
+  //      before that update.  The anchor is the fp32 global model at round start (the layout of
+  //      `master`).  prox_mu > 0 needs an anchor and no fused upload (else cudaErrorInvalidValue);
+  //      the reported loss stays the cross-entropy alone.
+  const float* prox_anchor = nullptr;
+  float prox_mu = 0.f;
 };
 cudaError_t mlp_round_sm100(const MlpRoundArgs& r, cudaStream_t stream);
 

@@ -10,6 +10,7 @@
 //   mc_val            committee validation: every member x every admitted candidate, one launch
 //   k_mc_consensus    scores, run_consensus<32>, ledger page, block record
 //   k_mc_fedavg       FedAvg of the selected masters into the global model and every client
+//                     (optionally followed by a server optimizer step: McServerOpt)
 #pragma once
 #include <cstdint>
 
@@ -114,7 +115,21 @@ cudaError_t mc_plan_round(const McArgs& a, cudaStream_t s);
 cudaError_t mc_byzantine(const McArgs& a, const int* ids, int n_ids, float scale, cudaStream_t s);
 // scores, sample counts and average costs come from the per-client constants in McClients
 cudaError_t mc_consensus(const McArgs& a, int weight_by_score, cudaStream_t s);
-cudaError_t mc_fedavg(const McArgs& a, int n_clients, cudaStream_t s);
+// Server-side optimizer of the FedOpt family (Reddi et al., 2021) applied per element to the
+// pseudo-gradient d = avg - g, g the current global model, after the FedAvg sum:
+//   momentum  m = fmaf(b1, m, d);                           g = fmaf(lr, m, g)
+//   adam      m = fmaf(b1, m, c1 * d); v = fmaf(b2, v, c2 * (d * d));      g = g + lr * m / (sqrtf(v) + tau)
+//   yogi      m as adam; d2 = d * d; v = v - c2 * d2 * sign(v - d2);       g as adam
+// c1 = 1 - b1, c2 = 1 - b2 of the fp32 b1, b2 (rounded to fp32 on the host), no bias correction; m starts at 0 and v
+// at tau^2 (the caller's buffers).  A round with nothing selected leaves g, m and v unchanged.
+enum McServerMode : int { MC_SERVER_NONE = 0, MC_SERVER_MOMENTUM = 1, MC_SERVER_ADAM = 2, MC_SERVER_YOGI = 3 };
+struct McServerOpt {
+  int mode = MC_SERVER_NONE;
+  float lr = 1.f, beta1 = 0.9f, beta2 = 0.99f, tau = 1e-3f;
+  float* m = nullptr;   // [n_params] fp32 server state: first moment (every mode but none)
+  float* v = nullptr;   // second moment (adam, yogi)
+};
+cudaError_t mc_fedavg(const McArgs& a, int n_clients, cudaStream_t s, const McServerOpt& so = McServerOpt{});
 // copy one blob to every client's blob slot (fp8: the quantised new global model)
 cudaError_t mc_broadcast_blob(const McArgs& a, const uint8_t* src, long long bytes, int n_clients,
                               cudaStream_t s);

@@ -193,10 +193,39 @@ __device__ __forceinline__ unsigned long long digest_term(float v, long long idx
          (static_cast<unsigned long long>(2 * idx + 1) * 0x9E3779B97F4A7C15ull);
 }
 
+// Server optimizer constants as the kernel uses them (c1, c2 rounded on the host).
+struct McServerK {
+  float lr, b1, b2, c1, c2, tau;
+  float* m; float* v;
+};
+
+// One element of the server step (mc_round.h): d = avg - g, state (m, v) updated in place,
+// returns the new global value.
+template <int MODE>
+__device__ __forceinline__ float server_step(const McServerK& k, float avg, float g, float& m, float& v) {
+  const float d = avg - g;
+  if (MODE == MC_SERVER_MOMENTUM) {
+    m = fmaf(k.b1, m, d);
+    return fmaf(k.lr, m, g);
+  }
+  m = fmaf(k.b1, m, k.c1 * d);
+  const float d2 = d * d;
+  if (MODE == MC_SERVER_ADAM) {
+    v = fmaf(k.b2, v, k.c2 * d2);
+  } else {   // yogi: sign(v - d2), sign(0) = 0
+    const float sg = v > d2 ? 1.f : (v < d2 ? -1.f : 0.f);
+    v = v - (k.c2 * d2) * sg;
+  }
+  return g + k.lr * m / (sqrtf(v) + k.tau);
+}
+
 // new_global = sum_k w_k * master_k over the selected clients in ascending id, one fp32 fma per
-// client per element (no atomics: bit-reproducible).  The result goes to the global model and to
-// every client's next-round work master / shadow.  The last block finishes the block record.
-__global__ void __launch_bounds__(kMcThreads) k_mc_fedavg(McArgs a, int n_clients) {
+// client per element (no atomics: bit-reproducible).  MODE != none: the average then takes the
+// server optimizer step from the current global model (mc_round.h).  The result goes to the
+// global model and to every client's next-round work master / shadow.  The last block finishes
+// the block record.  MODE is a template parameter so that plain FedAvg compiles as before.
+template <int MODE>
+__global__ void __launch_bounds__(kMcThreads) k_mc_fedavg(McArgs a, int n_clients, McServerK sk) {
   __shared__ const float4* src[kMcMaxClients];
   __shared__ float w[kMcMaxClients];
   __shared__ float4* dst_m[kMcMaxClients];
@@ -241,6 +270,18 @@ __global__ void __launch_bounds__(kMcThreads) k_mc_fedavg(McArgs a, int n_client
         const float wk = w[k];
         acc.x = fmaf(wk, v.x, acc.x); acc.y = fmaf(wk, v.y, acc.y);
         acc.z = fmaf(wk, v.z, acc.z); acc.w = fmaf(wk, v.w, acc.w);
+      }
+      if (MODE != MC_SERVER_NONE) {
+        const float4 g = g_f32[i];
+        float4 m = reinterpret_cast<const float4*>(sk.m)[i];
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (MODE != MC_SERVER_MOMENTUM) v = reinterpret_cast<const float4*>(sk.v)[i];
+        acc.x = server_step<MODE>(sk, acc.x, g.x, m.x, v.x);
+        acc.y = server_step<MODE>(sk, acc.y, g.y, m.y, v.y);
+        acc.z = server_step<MODE>(sk, acc.z, g.z, m.z, v.z);
+        acc.w = server_step<MODE>(sk, acc.w, g.w, m.w, v.w);
+        reinterpret_cast<float4*>(sk.m)[i] = m;
+        if (MODE != MC_SERVER_MOMENTUM) reinterpret_cast<float4*>(sk.v)[i] = v;
       }
     }
     dig += digest_term(acc.x, 4 * i) + digest_term(acc.y, 4 * i + 1) + digest_term(acc.z, 4 * i + 2) +
@@ -310,12 +351,25 @@ cudaError_t mc_consensus(const McArgs& a, int weight_by_score, cudaStream_t s) {
   return launch_pdl(k_mc_consensus, dim3(1), dim3(kMcThreads), 0, s, a, weight_by_score);
 }
 
-cudaError_t mc_fedavg(const McArgs& a, int n_clients, cudaStream_t s) {
+cudaError_t mc_fedavg(const McArgs& a, int n_clients, cudaStream_t s, const McServerOpt& so) {
   if (n_clients <= 0 || n_clients > kMcMaxClients || a.n_params % 4) return cudaErrorInvalidValue;
+  if (so.mode < MC_SERVER_NONE || so.mode > MC_SERVER_YOGI) return cudaErrorInvalidValue;
+  if (so.mode != MC_SERVER_NONE &&
+      (!(so.lr > 0.f) || !(so.beta1 >= 0.f && so.beta1 < 1.f) || !(so.beta2 >= 0.f && so.beta2 < 1.f) ||
+       !(so.tau > 0.f) || so.m == nullptr || (so.mode != MC_SERVER_MOMENTUM && so.v == nullptr)))
+    return cudaErrorInvalidValue;
+  McServerK sk{so.lr, so.beta1, so.beta2, static_cast<float>(1.0 - static_cast<double>(so.beta1)),
+               static_cast<float>(1.0 - static_cast<double>(so.beta2)), so.tau, so.m, so.v};
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const dim3 grid(mc_grid(a.n_params / 4, 4 * sms));
   note_launch();
-  return launch_pdl(k_mc_fedavg, dim3(mc_grid(a.n_params / 4, 4 * sms)), dim3(kMcThreads), 0, s, a, n_clients);
+  switch (so.mode) {
+    case MC_SERVER_MOMENTUM: return launch_pdl(k_mc_fedavg<MC_SERVER_MOMENTUM>, grid, dim3(kMcThreads), 0, s, a, n_clients, sk);
+    case MC_SERVER_ADAM: return launch_pdl(k_mc_fedavg<MC_SERVER_ADAM>, grid, dim3(kMcThreads), 0, s, a, n_clients, sk);
+    case MC_SERVER_YOGI: return launch_pdl(k_mc_fedavg<MC_SERVER_YOGI>, grid, dim3(kMcThreads), 0, s, a, n_clients, sk);
+    default: return launch_pdl(k_mc_fedavg<MC_SERVER_NONE>, grid, dim3(kMcThreads), 0, s, a, n_clients, sk);
+  }
 }
 
 cudaError_t mc_broadcast_blob(const McArgs& a, const uint8_t* src, long long bytes, int n_clients,

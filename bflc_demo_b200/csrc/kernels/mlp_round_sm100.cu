@@ -130,6 +130,8 @@ struct Args {
   // fused upload
   int has_fed; FedArgs f; long long upq_off[2];
   int n_samples, n_loss_terms, byz_mode; float byz_scale; int straggle_us;
+  // FedProx (PROX instantiations only): g' = mu (w - anchor) + g before the optimizer
+  const float* prox_anchor; float prox_mu;
 };
 
 struct Job {  // one output tile (bm rows x 64 columns)
@@ -306,16 +308,23 @@ __device__ __forceinline__ void mma_tile(const Job& j, uint8_t* smem, uint8_t* s
   ++pp.tile;
 }
 
-// SGD / Adam on n (<= 4) consecutive parameters starting at flat index pi, gradient in g[]:
+// SGD / Adam on n (<= 4) consecutive parameters starting at flat index pi, gradient in g0[]:
 // fp32 master, bf16 shadow (and the Adam moments) are updated in place; the new values are
 // returned in w[].  Coherent loads: other CTAs of this kernel wrote these buffers in earlier phases.
-__device__ __forceinline__ void opt_apply(const Args& a, long long pi, int n, const float* g,
+// PROX: the gradient becomes fmaf(mu, w - anchor, g) with w the master before this update (the
+// anchor is read-only for the whole launch).
+template <bool PROX>
+__device__ __forceinline__ void opt_apply(const Args& a, long long pi, int n, const float* g0,
                                           float bc1, float bc2, float (&w)[4]) {
-  float m[4], v[4];
+  float m[4], v[4], g[4], an[4];
   const bool vec = n == 4 && (pi & 3) == 0;
   if (vec) {
     const float4 w4 = __ldcg(reinterpret_cast<const float4*>(a.master + pi));
     w[0] = w4.x; w[1] = w4.y; w[2] = w4.z; w[3] = w4.w;
+    if (PROX) {
+      const float4 a4 = __ldg(reinterpret_cast<const float4*>(a.prox_anchor + pi));
+      an[0] = a4.x; an[1] = a4.y; an[2] = a4.z; an[3] = a4.w;
+    }
     if (a.adam) {
       const float4 m4 = __ldcg(reinterpret_cast<const float4*>(a.adam_m + pi));
       const float4 v4 = __ldcg(reinterpret_cast<const float4*>(a.adam_v + pi));
@@ -325,12 +334,14 @@ __device__ __forceinline__ void opt_apply(const Args& a, long long pi, int n, co
   } else {
     for (int k = 0; k < n; ++k) {
       w[k] = __ldcg(a.master + pi + k);
+      if (PROX) an[k] = __ldg(a.prox_anchor + pi + k);
       if (a.adam) { m[k] = __ldcg(a.adam_m + pi + k); v[k] = __ldcg(a.adam_v + pi + k); }
     }
   }
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     if (k >= n) break;
+    g[k] = PROX ? fmaf(a.prox_mu, w[k] - an[k], g0[k]) : g0[k];
     if (a.adam) {
       m[k] = a.beta1 * m[k] + (1.f - a.beta1) * g[k];
       v[k] = a.beta2 * v[k] + (1.f - a.beta2) * g[k] * g[k];
@@ -366,8 +377,9 @@ __device__ __forceinline__ int rows_per_quarter(int bm) { return bm == 64 ? 16 :
 // without the prefetch: +4.3 us per step, measured).  fp8 mode: the updated tile is parked in
 // the staging buffer and re-quantised one K-group (32 columns of a row) per thread.  On the last
 // step the values (optionally Byzantine-transformed) also go to the upload buffers the committee
-// and the FedAvg kernel read.
-template <bool FP8>
+// and the FedAvg kernel read.  PROX: the anchor's float4s are prefetched with the master (same
+// reason) and the gradient becomes fmaf(mu, w - anchor, g) before SGD / Adam.
+template <bool FP8, bool PROX>
 __device__ __forceinline__ void epilogue_opt(const Job& j, const Args& a, int q, int half, int lane,
                                              uint64_t* accum_bar, uint32_t tmem_base, float* stg,
                                              Pipe& pp) {
@@ -378,13 +390,15 @@ __device__ __forceinline__ void epilogue_opt(const Job& j, const Args& a, int q,
   const int nc = j.n0 + half * 32;               // this warp's 32 columns
   const long long pbase = reinterpret_cast<float*>(j.d) - a.master;
   const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + half * 32;
-  float4 wpre[8], mpre[8], vpre[8];
+  float4 wpre[8], mpre[8], vpre[8], apre[8];
 #pragma unroll
   for (int it = 0; it < 8; ++it) {
     const int rw = row_base + it * 4 + cr, col = nc + cg;
     const bool ok = it < n_it && rw < j.M && col + 3 < j.N;
     const long long pi = pbase + static_cast<long long>(rw) * j.ldd + col;
     wpre[it] = ok ? __ldcg(reinterpret_cast<const float4*>(a.master + pi)) : make_float4(0.f, 0.f, 0.f, 0.f);
+    if (PROX)
+      apre[it] = ok ? __ldg(reinterpret_cast<const float4*>(a.prox_anchor + pi)) : make_float4(0.f, 0.f, 0.f, 0.f);
     if (a.adam) {
       mpre[it] = ok ? __ldcg(reinterpret_cast<const float4*>(a.adam_m + pi)) : make_float4(0.f, 0.f, 0.f, 0.f);
       vpre[it] = ok ? __ldcg(reinterpret_cast<const float4*>(a.adam_v + pi)) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -416,8 +430,13 @@ __device__ __forceinline__ void epilogue_opt(const Job& j, const Args& a, int q,
       const long long pi = pbase + static_cast<long long>(rw) * j.ldd + col;
       float4 w = make_float4(0.f, 0.f, 0.f, 0.f);
       if (valid) {
-        const float4 g = *reinterpret_cast<const float4*>(stg + rr * kStgLd + cg);
+        float4 g = *reinterpret_cast<const float4*>(stg + rr * kStgLd + cg);
         w = wpre[it];
+        if (PROX) {
+          const float mu = a.prox_mu;
+          g.x = fmaf(mu, w.x - apre[it].x, g.x); g.y = fmaf(mu, w.y - apre[it].y, g.y);
+          g.z = fmaf(mu, w.z - apre[it].z, g.z); g.w = fmaf(mu, w.w - apre[it].w, g.w);
+        }
         if (a.adam) {
           float4 m = mpre[it], s = vpre[it];
           const float b1 = a.beta1, b2 = a.beta2, c1 = 1.f - a.beta1, c2 = 1.f - a.beta2;
@@ -474,7 +493,7 @@ __device__ __forceinline__ void epilogue_opt(const Job& j, const Args& a, int q,
 }
 
 // epilogue warps 4..11: q = TMEM lane quarter, half = which 32 of the tile's 64 columns
-template <bool FP8>
+template <bool FP8, bool PROX>
 __device__ __forceinline__ void epilogue_tile(const Job& j, const Args& a, int q, int half, int lane,
                                               uint64_t* accum_bar, uint32_t tmem_base,
                                               float* stg, float* sbias, Pipe& pp) {
@@ -485,7 +504,7 @@ __device__ __forceinline__ void epilogue_tile(const Job& j, const Args& a, int q
     epi_bar();
   }
   if (j.mode == E_OPT) {
-    epilogue_opt<FP8>(j, a, q, half, lane, accum_bar, tmem_base, stg, pp);
+    epilogue_opt<FP8, PROX>(j, a, q, half, lane, accum_bar, tmem_base, stg, pp);
     return;
   }
   const int rpq = rows_per_quarter(j.bm);
@@ -979,7 +998,9 @@ __device__ __forceinline__ void grid_barrier(unsigned int* counter, unsigned int
   ptx::tc_fence_after_sync();
 }
 
-template <bool FP8>
+// PROX: FedProx term in every optimizer update.  A template parameter, not a runtime branch, so
+// that the default instantiations keep their register allocation.
+template <bool FP8, bool PROX>
 __global__ void __launch_bounds__(kThreads, 1)
 mlp_round_kernel(const __grid_constant__ Maps maps, const Args a) {
   extern __shared__ uint8_t smem_raw[];
@@ -1044,7 +1065,7 @@ mlp_round_kernel(const __grid_constant__ Maps maps, const Args a) {
   constexpr bool EPI = decltype(epi_tag)::value;
   auto run = [&](const Job& j) {
     if constexpr (EPI) {
-      epilogue_tile<FP8>(j, a, q, half, lane, accum_bar, tmem_base, stg, sbias, pp);
+      epilogue_tile<FP8, PROX>(j, a, q, half, lane, accum_bar, tmem_base, stg, sbias, pp);
     } else {
       if (warp == 0) produce_tile<FP8>(j, smem, sf_smem, full_bar, empty_bar, pp);
       else if (warp == 1) mma_tile<FP8>(j, smem, sf_smem, full_bar, empty_bar, accum_bar, tmem_base, pp);
@@ -1188,7 +1209,7 @@ mlp_round_kernel(const __grid_constant__ Maps maps, const Args a) {
         *gp = 0.f;
         float w[4];
         const long long pi = gp - a.grad;
-        opt_apply(a, pi, 1, &g, bc1, bc2, w);
+        opt_apply<PROX>(a, pi, 1, &g, bc1, bc2, w);
         if (up) {
           float wu = w[0];
           if (ud.global != nullptr) { const float g0 = __ldcg(ud.global + pi); wu = g0 - ud.byz_scale * (wu - g0); }
@@ -1210,7 +1231,7 @@ mlp_round_kernel(const __grid_constant__ Maps maps, const Args a) {
         const float4 g4 = __ldcg(reinterpret_cast<const float4*>(a.grad) + i);
         const float g[4] = {g4.x, g4.y, g4.z, g4.w};
         float w[4];
-        opt_apply(a, 4 * i, 4, g, bc1, bc2, w);
+        opt_apply<PROX>(a, 4 * i, 4, g, bc1, bc2, w);
         reinterpret_cast<float4*>(a.grad)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
     }
@@ -1311,6 +1332,10 @@ cudaError_t mlp_round_sm100(const MlpRoundArgs& r, cudaStream_t stream) {
               !r.h_q || !r.h_sf))
     return cudaErrorNotSupported;
   if (r.fed != nullptr && !epiopt) return cudaErrorNotSupported;
+  // FedProx needs its anchor; it is not combined with the fused upload (one client per GPU)
+  if (!(r.prox_mu >= 0.f) || (r.prox_mu > 0.f && (r.prox_anchor == nullptr || r.fed != nullptr)))
+    return cudaErrorInvalidValue;
+  const bool prox = r.prox_mu > 0.f;
   // weight-gradient tiles: 64 rows (UMMA M = 64) spread the optimizer epilogue over twice the CTAs;
   // BFLC_MLP_BMW=128 keeps the 128-row tiles
   static const int bmw_env = [] { const char* e = std::getenv("BFLC_MLP_BMW"); return e && std::atoi(e) == 128 ? 128 : 64; }();
@@ -1372,17 +1397,19 @@ cudaError_t mlp_round_sm100(const MlpRoundArgs& r, cudaStream_t stream) {
   a.upq_off[0] = r.upq_off[0]; a.upq_off[1] = r.upq_off[1];
   a.n_samples = r.n_samples; a.n_loss_terms = r.n_loss_terms; a.byz_mode = r.byz_mode; a.byz_scale = r.byz_scale;
   a.straggle_us = r.straggle_us;
+  a.prox_anchor = prox ? r.prox_anchor : nullptr; a.prox_mu = prox ? r.prox_mu : 0.f;
 
-  static bool configured[2] = {false, false};
-  if (!configured[fp8 ? 1 : 0]) {
-    e = fp8 ? cudaFuncSetAttribute(mlp_round_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal)
-            : cudaFuncSetAttribute(mlp_round_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
+  auto kern = fp8 ? (prox ? mlp_round_kernel<true, true> : mlp_round_kernel<true, false>)
+                  : (prox ? mlp_round_kernel<false, true> : mlp_round_kernel<false, false>);
+  static bool configured[4] = {false, false, false, false};
+  const int ki = (fp8 ? 1 : 0) + (prox ? 2 : 0);
+  if (!configured[ki]) {
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
     if (e != cudaSuccess) return e;
-    configured[fp8 ? 1 : 0] = true;
+    configured[ki] = true;
   }
   note_launch();
-  if (fp8) return launch_pdl(mlp_round_kernel<true>, dim3(grid), dim3(kThreads), kSmemTotal, stream, m, a);
-  return launch_pdl(mlp_round_kernel<false>, dim3(grid), dim3(kThreads), kSmemTotal, stream, m, a);
+  return launch_pdl(kern, dim3(grid), dim3(kThreads), kSmemTotal, stream, m, a);
 }
 
 }  // namespace bflc

@@ -76,6 +76,7 @@ _ROUND_STATE = struct.Struct("<4I8I8fIfQII")
 class FusedEngine:
     def __init__(self, cfg: FLConfig, shard: Shard, *, rank: int = 0, world: int = 1,
                  device: int = 0, group=None, in_dim: Optional[int] = None):
+        cfg.require_plain_fedavg("FusedEngine")
         assert cfg.clients == world, "one client per rank"
         assert world <= 8
         self.cfg, self.rank, self.world, self.device = cfg, rank, world, device

@@ -56,6 +56,7 @@ class GenericFedEngine:
 
     def __init__(self, cfg: FLConfig, net: FlatNet, shard: Shard, *, rank: int = 0, world: int = 1,
                  device: int = 0, group=None):
+        cfg.require_plain_fedavg("GenericFedEngine")
         assert cfg.clients == world and world <= 8
         self.cfg, self.net, self.rank, self.world, self.device = cfg, net, rank, world, device
         self.group = group

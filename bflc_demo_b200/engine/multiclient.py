@@ -26,6 +26,13 @@ S_c = (rows_c // B) * B samples in steps_c = S_c / B * local_epochs steps, valid
 member on n_val_c = min(val_samples or rows_c, rows_c) rows of its own shard and reports
 n_samples = S_c, so FedAvg weights the selected clients by their sample counts -- the rule
 ``FusedEngine`` applies per rank.  These constants live in the device-resident ``McClients``.
+
+Against client drift under skewed data (DESIGN.md, "FedProx and server optimizers"):
+``cfg.prox_mu`` > 0 adds the FedProx term mu/2 ||w - w_global||^2 to every client's local loss (the
+anchor is ``global_master``, which holds the round-start model for the whole training phase), and
+``cfg.server_optimizer`` (momentum | adam | yogi) turns the FedAvg step into a server optimizer
+step on the pseudo-gradient average - global, with its state in ``server_m`` / ``server_v``.  The
+committee, the election, the FedAvg weights and the host ledger are the same in every setting.
 """
 from __future__ import annotations
 
@@ -145,13 +152,25 @@ class MultiClientEngine:
         self.correct = plan_view("mc_plan_correct_off", MAX_CLIENTS * MAX_CLIENTS, torch.int32).view(
             MAX_CLIENTS, MAX_CLIENTS)
 
-        # ---- one persistent trainer per client (own barrier word, step base, Adam moments) ---
+        # ---- server optimizer state: m = 0, v = tau^2 at genesis (Reddi et al., Algorithm 2) ---
+        so = cfg.server_optimizer
+        self.server_m = torch.zeros(P, device=dev, dtype=torch.float32) if so != "none" else None
+        self.server_v = (torch.full((P,), cfg.server_tau * cfg.server_tau, device=dev, dtype=torch.float32)
+                         if so in ("adam", "yogi") else None)
+        self.server_kw = dict(server_optimizer=so, lr=cfg.server_lr, beta1=cfg.server_beta1,
+                              beta2=cfg.server_beta2, tau=cfg.server_tau,
+                              m=self.server_m.data_ptr() if self.server_m is not None else 0,
+                              v=self.server_v.data_ptr() if self.server_v is not None else 0)
+
+        # ---- one persistent trainer per client (own barrier word, step base, Adam moments);
+        #      FedProx anchors every client to the round-start global model
         self.trainers: List[FlatMLP] = []
         for c in range(n):
             tr = FlatMLP(self.spec, self.master[c], self.shadow[c], self.grad[c], B,
                          optimizer=cfg.optimizer, lr=cfg.learning_rate,
                          loss_sum=self.loss_sum[c:c + 1], correct=self.train_correct[c:c + 1],
-                         step_dev_ptr=pp + sz["mc_plan_opt_step_off"] + 4 * c, fp8=self.fp8)
+                         step_dev_ptr=pp + sz["mc_plan_opt_step_off"] + 4 * c, fp8=self.fp8,
+                         prox_mu=cfg.prox_mu, prox_anchor=self.global_master if cfg.prox_mu > 0 else None)
             if not tr.fused_ok(self.steps_per_client[c]):
                 raise ValueError("shape outside the persistent trainer's limits")
             self.trainers.append(tr)
@@ -261,12 +280,17 @@ class MultiClientEngine:
                  self.in_dim, self.cfg.hidden, self.n_classes, self.max_cand, self.cfg.committee_size, self.fp8)
 
     def phase_aggregate(self):
-        """Consensus, ledger page, block record, FedAvg into the global model and every client."""
+        """Consensus, ledger page, block record, FedAvg (+ server optimizer step) into the global
+        model and every client."""
         m, cfg = self.mod, self.cfg
         m.mc_consensus(self.args, cfg.weight_by_score)
-        m.mc_fedavg(self.args, cfg.clients)
+        self.fedavg()
         if self.fp8:
             self._broadcast_global_blob()
+
+    def fedavg(self):
+        """The FedAvg kernel alone, with this engine's server optimizer."""
+        self.mod.mc_fedavg(self.args, self.cfg.clients, **self.server_kw)
 
     def _enqueue_round(self):
         n0 = self.mod.launch_count()

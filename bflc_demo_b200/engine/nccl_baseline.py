@@ -37,6 +37,7 @@ from .fused import ROLE_COMM, ROLE_TRAINER, initial_roles
 class NcclBaselineEngine:
     def __init__(self, cfg: FLConfig, shard: Shard, *, rank: int = 0, world: int = 1,
                  device: int = 0, group=None, broadcast: bool = False):
+        cfg.require_plain_fedavg("NcclBaselineEngine")
         self.cfg, self.rank, self.world, self.group = cfg, rank, world, group
         self.dev = torch.device("cuda", device)
         torch.cuda.set_device(device)

@@ -44,12 +44,24 @@ def softmax_regression_spec(n_features: int = 5, n_class: int = 2) -> ParamSpec:
 
 class FlatMLP:
     """Fused-kernel trainer over flat buffers.  ``master``/``shadow``/``grad`` are 1-D tensors
-    of ``spec.total`` elements (fp32 / bf16 / fp32); they may live in the symmetric heap."""
+    of ``spec.total`` elements (fp32 / bf16 / fp32); they may live in the symmetric heap.
+
+    ``prox_mu`` > 0 (FedProx): every step adds ``prox_mu * (w - prox_anchor)`` to the gradient, the
+    gradient of ``prox_mu / 2 * ||w - prox_anchor||^2``.  ``prox_anchor`` is an fp32 tensor with the
+    master's layout (the global model at round start) that stays fixed while the trainer runs.  The
+    reported loss stays the cross-entropy alone."""
 
     def __init__(self, spec: ParamSpec, master: torch.Tensor, shadow: torch.Tensor,
                  grad: torch.Tensor, batch: int, *, optimizer: str = "sgd", lr: float = 1e-3,
                  loss_sum: Optional[torch.Tensor] = None, correct: Optional[torch.Tensor] = None,
-                 step_dev_ptr: int = 0, fp8: bool = False):
+                 step_dev_ptr: int = 0, fp8: bool = False, prox_mu: float = 0.0,
+                 prox_anchor: Optional[torch.Tensor] = None):
+        if prox_mu < 0 or (prox_mu > 0 and prox_anchor is None):
+            raise ValueError("prox_mu must be >= 0, and prox_mu > 0 needs a prox_anchor")
+        if prox_anchor is not None and (prox_anchor.shape != master.shape or prox_anchor.dtype != torch.float32):
+            raise ValueError("prox_anchor: fp32 with the master's shape")
+        self.prox_mu = float(prox_mu)
+        self.prox_anchor = prox_anchor if self.prox_mu > 0 else None
         self.spec, self.master, self.shadow, self.grad = spec, master, shadow, grad
         self.p = spec.views(master)
         self.s = spec.views(shadow)
@@ -122,6 +134,8 @@ class FlatMLP:
         B = self.batch
         for i in range(steps):
             self.forward_backward(X[i * B:(i + 1) * B], Y[i * B:(i + 1) * B])
+            if self.prox_mu > 0:
+                self.grad.add_(self.master - self.prox_anchor, alpha=self.prox_mu)
             self.optimizer_step(i + 1)
 
     def fused_ok(self, steps: int) -> bool:
@@ -171,7 +185,8 @@ class FlatMLP:
                       x_q if self.fp8 else None, x_sf if self.fp8 else None,
                       self.work_q if self.fp8 else None, self.h_q if self.fp8 else None,
                       self.h_sf if self.fp8 else None, fed, list(upq_off), n_samples, n_loss_terms,
-                      byz_mode, byz_scale, straggle_us)
+                      byz_mode, byz_scale, straggle_us, prox_mu=self.prox_mu,
+                      prox_anchor=self.prox_anchor)
 
     # ------------------------------------------------------------ evaluation
     def accuracy_counts(self, X: torch.Tensor, Y: torch.Tensor, shadow: Optional[torch.Tensor] = None,

@@ -4,6 +4,8 @@ reference, python-sdk/main.py:343-358, for one NVSwitch box):
     python -m bflc_demo_b200.run --model mlp --rounds 20                       # 1 GPU, solo
     python -m bflc_demo_b200.run --clients 20 --rounds 20     # 20 clients on 1 GPU (20/4/10/6)
     python -m bflc_demo_b200.run --clients 20 --alpha 0.5 --size-sigma 0.8    # skewed labels + sizes
+    python -m bflc_demo_b200.run --clients 20 --alpha 0.1 --prox-mu 0.01 --server-opt adam \
+        --server-lr 0.01                                  # FedProx clients + FedAdam server
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 \\
         -m bflc_demo_b200.run --model resnet18 --rounds 5 --byzantine 7       # config #4
 
@@ -55,7 +57,24 @@ def main(argv=None):
     ap.add_argument("--size-sigma", type=float, default=0.0,
                     help="--clients: log-normal spread of the shard sizes (0 = equal shards; the "
                          "total stays clients x samples)")
+    fo = ap.add_argument_group("FedProx and server optimizers (--clients only)")
+    fo.add_argument("--prox-mu", type=float, default=None,
+                    help="FedProx: add mu/2 ||w - w_global||^2 to every client's local loss (default 0)")
+    fo.add_argument("--server-opt", default=None, choices=["none", "momentum", "adam", "yogi"],
+                    help="server step on the pseudo-gradient average - global (default none = FedAvg)")
+    fo.add_argument("--server-lr", type=float, default=None, help="server learning rate (default 1.0)")
+    fo.add_argument("--server-beta1", type=float, default=None, help="default 0.9")
+    fo.add_argument("--server-beta2", type=float, default=None, help="default 0.99")
+    fo.add_argument("--server-tau", type=float, default=None, help="adaptivity (default 1e-3)")
     a = ap.parse_args(argv)
+    fedopt = {k: v for k, v in (("prox_mu", a.prox_mu), ("server_optimizer", a.server_opt),
+                                 ("server_lr", a.server_lr), ("server_beta1", a.server_beta1),
+                                 ("server_beta2", a.server_beta2), ("server_tau", a.server_tau))
+              if v is not None}
+    if fedopt and a.clients < 2:
+        ap.error("--prox-mu and --server-* need --clients N (N >= 2): only the multi-client engine "
+                 "implements FedProx and the server optimizers")
+    a.fedopt = fedopt
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -133,7 +152,7 @@ def run_multiclient(a):
     cfg = FLConfig(clients=a.clients, committee_size=a.committee, needed_updates=a.needed,
                    aggregate_count=a.aggregate, batch_size=B, samples_per_client=S, learning_rate=LR,
                    optimizer=a.optimizer, byzantine_ranks=a.byzantine, ring_slots=1024,
-                   dtype=a.dtype, non_iid_alpha=a.alpha).validate()
+                   dtype=a.dtype, non_iid_alpha=a.alpha, **a.fedopt).validate()
     # shard sizes in whole batches (every client trains at least one; fp8 batches are 128-row tiles)
     sizes = client_sizes(a.clients, S, sigma=a.size_sigma, multiple=B, seed=7) if a.size_sigma > 0 else None
     shards = femnist_like(a.clients, S, seed=7, alpha=cfg.non_iid_alpha, sizes=sizes)
@@ -141,6 +160,8 @@ def run_multiclient(a):
     eng = MultiClientEngine(cfg, shards, device=0)
     print(f"[clients] alpha {cfg.non_iid_alpha} size_sigma {a.size_sigma} rows per client "
           f"{eng.rows_per_client}")
+    print(f"[clients] prox_mu {cfg.prox_mu} server_optimizer {cfg.server_optimizer} server_lr {cfg.server_lr} "
+          f"server_beta1 {cfg.server_beta1} server_beta2 {cfg.server_beta2} server_tau {cfg.server_tau}")
     eng.capture()
     log = RunLog(rank=0)
     timer = PhaseTimer()
@@ -153,7 +174,9 @@ def run_multiclient(a):
                   committee=[r for r, x in enumerate(st["roles"]) if x & 2])
     errs = eng.drain_blocks()
     summary = dict(rounds=a.rounds, clients=a.clients, alpha=cfg.non_iid_alpha, size_sigma=a.size_sigma,
-                   rows_per_client=eng.rows_per_client, wall_s=round(time.time() - t0, 3),
+                   rows_per_client=eng.rows_per_client, prox_mu=cfg.prox_mu,
+                   server_optimizer=cfg.server_optimizer, server_lr=cfg.server_lr, server_beta1=cfg.server_beta1,
+                   server_beta2=cfg.server_beta2, server_tau=cfg.server_tau, wall_s=round(time.time() - t0, 3),
                    timing=timer.summary(), ledger_mismatches=errs, chain_ok=eng.host_ledger.verify_chain(),
                    blocks=eng.host_ledger.n_blocks(), launches_per_round=eng.launches_per_round)
     print("SUMMARY " + json.dumps(summary))

@@ -1,7 +1,7 @@
 """Rounds/s of the multi-client engine (engine/multiclient.py) on one GPU.
 
     python scripts/bench_multiclient.py [--clients 8 20 32] [--skewed 20] [--size-sigma 0.8]
-                                        [--steps 20] [--warmup 5]
+                                        [--fedopt 20] [--repeat 1] [--steps 20] [--warmup 5]
 
 For C clients (committee / needed / aggregate in the reference's 20 / 4 / 10 / 6 proportions),
 4096 samples and batch 512 per client, fp8 + Adam and bf16 + SGD: device-event time of the
@@ -12,6 +12,11 @@ alone against the HBM roofline.  Prints one JSON line per configuration.
 ``--skewed C``: the same C-client workload with unequal shards -- log-normal sizes
 (``client_sizes``, ``--size-sigma``) in whole batches with the same total sample count (C x 4096),
 so training time is comparable; the validation grid spans the largest member's rows.
+
+``--fedopt C``: the equal-shard C-client workload with FedProx clients (prox_mu 0.01) and a FedAdam
+server (server_optimizer adam), to compare its train / validate / consensus + FedAvg split row
+against row with the plain rows.  ``--repeat N`` runs the whole list N times, interleaved, which
+shows the run-to-run spread.
 """
 from __future__ import annotations
 
@@ -56,10 +61,14 @@ def timed(fn, flush, reps, stream):
     return ts[len(ts) // 2]
 
 
-def bench(clients, dtype, opt, steps, warmup, flush, size_sigma=0.0):
+FEDOPT = dict(prox_mu=0.01, server_optimizer="adam", server_lr=0.01)
+
+
+def bench(clients, dtype, opt, steps, warmup, flush, size_sigma=0.0, fedopt=None):
     cfg = FLConfig.reference_scaled(clients, model="mlp", dataset="femnist", hidden=256, batch_size=512,
                                     samples_per_client=4096, dtype=dtype, optimizer=opt,
-                                    learning_rate=0.002 if opt == "adam" else 0.05, ring_slots=1024)
+                                    learning_rate=0.002 if opt == "adam" else 0.05, ring_slots=1024,
+                                    **(fedopt or {}))
     sizes = client_sizes(clients, 4096, sigma=size_sigma, multiple=512, seed=7) if size_sigma > 0 else None
     eng = MultiClientEngine(cfg, femnist_like(clients, 4096, seed=7, sizes=sizes), device=0)
     eng.capture()
@@ -93,16 +102,19 @@ def bench(clients, dtype, opt, steps, warmup, flush, size_sigma=0.0):
     # FedAvg alone (last: it re-averages the already averaged masters, the ledger is not drained again)
     g = torch.cuda.CUDAGraph()
     with torch.cuda.graph(g, stream=s):
-        eng.mod.mc_fedavg(eng.args, clients)
+        eng.fedavg()
     with torch.cuda.stream(s):
         g.replay()
     fedavg_us = timed(lambda: g.replay(), flush, steps, s)
     P = eng.n_params
     fed_bytes = n_sel * P * 4 + P * 6 + clients * P * 6
+    # server optimizer: reads the current global model, reads and writes m (and v)
+    fed_bytes += {"none": 0, "momentum": 3, "adam": 5, "yogi": 5}[cfg.server_optimizer] * P * 4
     rows = eng.rows_per_client
     return dict(clients=clients, committee=cfg.committee_size, needed=cfg.needed_updates,
                 aggregate=cfg.aggregate_count, dtype=dtype, optimizer=opt, samples=4096, batch=512,
-                size_sigma=size_sigma, samples_total=sum(rows), rows_min=min(rows), rows_max=max(rows),
+                size_sigma=size_sigma, prox_mu=cfg.prox_mu, server_optimizer=cfg.server_optimizer,
+                samples_total=sum(rows), rows_min=min(rows), rows_max=max(rows),
                 round_us=round(round_us, 1), rounds_per_s=round(1e6 / round_us, 1),
                 train_us=round(split[0], 1), validate_us=round(split[1], 1),
                 consensus_fedavg_us=round(split[2], 1), fedavg_us=round(fedavg_us, 1),
@@ -118,15 +130,20 @@ def main():
     ap.add_argument("--skewed", type=int, nargs="*", default=[20],
                     help="client counts also run with unequal shards (--size-sigma)")
     ap.add_argument("--size-sigma", type=float, default=0.8)
+    ap.add_argument("--fedopt", type=int, nargs="*", default=[20],
+                    help="client counts also run with FedProx + FedAdam (%s)" % FEDOPT)
+    ap.add_argument("--repeat", type=int, default=1, help="run the whole list this many times")
     a = ap.parse_args()
     print(json.dumps(dict(gpu=torch.cuda.get_device_name(0), power_limit=power_limit(),
                           hbm_peak_bytes_per_s=HBM_PEAK)), flush=True)
     flush = torch.empty(256 << 20, device="cuda", dtype=torch.uint8)   # > L2
-    runs = [(c, 0.0) for c in a.clients] + [(c, a.size_sigma) for c in a.skewed]
-    for c, sigma in runs:
-        for dtype, opt in (("fp8", "adam"), ("bf16", "sgd")):
-            print(json.dumps(bench(c, dtype, opt, a.steps, a.warmup, flush, sigma)), flush=True)
-            torch.cuda.empty_cache()
+    runs = ([(c, 0.0, None) for c in a.clients] + [(c, a.size_sigma, None) for c in a.skewed] +
+            [(c, 0.0, FEDOPT) for c in a.fedopt])
+    for _ in range(a.repeat):
+        for c, sigma, fo in runs:
+            for dtype, opt in (("fp8", "adam"), ("bf16", "sgd")):
+                print(json.dumps(bench(c, dtype, opt, a.steps, a.warmup, flush, sigma, fo)), flush=True)
+                torch.cuda.empty_cache()
 
 
 if __name__ == "__main__":
